@@ -10,9 +10,11 @@ sum pooling -- hyper_params.py:15) forward + nll_loss + backward [+ gradient all
 `value`   : inputs (raw graphs) resident in HBM, L2 flushed between steps, device-timed, max over ranks.
 `e2e`     : same step through ClassificationPipeline.step(): pinned host buffers -> H2D -> ... -> loss D2H.
 `roofline`: the aggregation kernel (dn4gl_spmm_sum_f32 at D=32), algorithmic bytes / CUDA-event duration.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  `--dump-outputs DIR` also writes what the last timed step handed back (loss, updated
+parameters, their gradients, BatchNorm statistics) as DIR/<name>.npy, so that two builds can be compared output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -23,6 +25,7 @@ from argparse import Namespace
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # leave the source tree as it is (it may be read-only)
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -45,7 +48,30 @@ def parse():
     ap.add_argument("--no-size-hints", dest="size_hints", action="store_false",
                     help="let the transform read its output sizes back from the device (one device->host sync per step) "
                          "instead of taking transforms.tu_conjugate_sizes(raw) from the host batch")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+    return a
+
+
+def dump_outputs(out_dir, loss, model):
+    """what a caller of the timed step holds after it: the returned loss and the model the step updated in place -- every
+    parameter, the gradient this step computed for it, the BatchNorm running statistics.  Inputs and initial weights
+    are seeded, so the same arguments give the same arrays up to floating-point reordering."""
+    arrays = {"loss": loss}
+    for n, p in model.named_parameters():
+        arrays["param." + n] = p
+        if p.grad is not None:
+            arrays["grad." + n] = p.grad
+    for n, b in model.named_buffers():
+        if b.is_floating_point():
+            arrays["buffer." + n] = b
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.detach().float().cpu().numpy())
 
 
 def measured_peaks():
@@ -347,6 +373,11 @@ class ClockSampler:
                                        "-lms", "50"], stdout=self.f, stderr=subprocess.DEVNULL)
         except Exception:   # noqa: BLE001
             self.p = None
+        atexit.register(self._kill)      # an exception before stop() must not leave the sampler running
+
+    def _kill(self):
+        if self.p is not None and self.p.poll() is None:
+            self.p.kill()
 
     def mark_start(self):
         self.t0 = time.time()
@@ -503,6 +534,8 @@ def ours(a):
     final_loss = float(loss.item())      # read NOW: `loss` is the captured step's static buffer, later steps overwrite it
     m1 = nmalloc()
     ms = max_over_ranks(e0.elapsed_time(e1), dev) / a.steps
+    if a.dump_outputs and rank == 0:      # before the loops below step the model again
+        dump_outputs(a.dump_outputs, loss, model)
     # what the in-loop L2 flush costs: the same K steps without it, and K flushes alone (informational -- `value` and
     # `ms_per_step` above are the flushed loop, flush included)
     ex0, ex1, ex2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))

@@ -1,6 +1,6 @@
 """Generate tests/golden/* by executing the UNMODIFIED reference under oracle/shims.
 
-Run in the build container only (needs /root/reference):   python -m oracle.gen_golden
+Needs a checkout of the original project:   DN4GL_REFERENCE_ROOT=<checkout> python -m oracle.gen_golden
 The fixtures pin (a) the transforms' exact index outputs and (b) forward values, loss and every parameter
 gradient of the reference's own GIN / RGIN(cls) / RGIN / DMPNN classes on small seeded batches.  They travel
 to the GPU box; nothing else of the reference does.
@@ -20,6 +20,20 @@ from . import ref_drive as rd
 from . import transforms as OT
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+
+
+def _save(out, name):
+    """one file per key under tests/golden/<name>/ (the key's "/" become directories): every file stays small"""
+    for k, v in out.items():
+        path = os.path.join(OUT, name, k + ".pt")
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        th.save(v, path)
+
+
+def _load(name):
+    root = os.path.join(OUT, name)
+    return {os.path.relpath(os.path.join(d, f), root)[:-3]: th.load(os.path.join(d, f), weights_only=False)
+            for d, _, files in os.walk(root) for f in files if f.endswith(".pt")}
 
 
 def _np(d):
@@ -55,15 +69,14 @@ def gen_transforms():
     for base in (dict(add_rev=False, add_dummy=True, convert_conj=False), dict(add_rev=True, add_dummy=True, convert_conj=True)):
         c = dict(synth.counting_config("small"), **base)
         out["cfg/%s" % "-".join("%s%d" % (k[:5], v) for k, v in base.items())] = dict(inp=c, out=rd.ref_process_model_config(c))
-    th.save(out, os.path.join(OUT, "transforms.pt"))
+    _save(out, "transforms")
     print("transforms.pt:", list(out))
 
 
 def gen_augment():
     """SURVEY.md 8(f) rank 3: the reference's remove_loops / add_reversed_edges / calculate_norms /
     calculate_eigenvalues (train.py:270-345, 500-527) on seeded batches, added to transforms.pt."""
-    path = os.path.join(OUT, "transforms.pt")
-    out = th.load(path, weights_only=False)
+    out = _load("transforms")
     for shape, bs, seed in (("small", 6, 23), ("large", 1, 24)):
         p, g, _ = synth.counting_batch(shape, bs, seed=seed)
         cfg = synth.counting_config(shape)
@@ -80,15 +93,14 @@ def gen_augment():
             cfg=cfg, pattern=_np(p), graph=_np(g), pattern_loops=_np(loops["pattern"]), graph_loops=_np(loops["graph"]),
             pattern_noloops=lp, graph_noloops=lg, pattern_rev=rp, graph_rev=rg, pattern_rev_dummy=dp, graph_rev_dummy=dg,
             norms_self_loop=rd.ref_sub_norms_eigen(dg, True), norms_no_self_loop=rd.ref_sub_norms_eigen(dg, False))
-    th.save(out, path)
+    _save(out, "transforms")
     print("transforms.pt:", list(out))
 
 
 def gen_match_weights():
     """SURVEY.md 8(f) rank 2: the reference's numba loops compute_nodeseq_subisoweights / compute_edgeseq_subisoweights
     (dataset.py:54-108) driven as calculate_node_weights / calculate_edge_weights do (:1491-1520), added to transforms.pt."""
-    path = os.path.join(OUT, "transforms.pt")
-    out = th.load(path, weights_only=False)
+    out = _load("transforms")
     for shape, bs, seed in (("small", 16, 61), ("large", 2, 62)):
         p, g, _ = synth.counting_batch(shape, bs, seed=seed)
         mats = synth.random_subisomorphisms(p, g, seed=seed)
@@ -108,7 +120,7 @@ def gen_match_weights():
     nw, ew = rd.ref_match_weights(mats, p, g)
     out["match/runs"] = dict(pattern=_np(p), graph=_np(g), mats=mats, node_weights=nw, edge_weights=ew,
                              conj=rd.ref_conjugate_subisomorphisms(mats, p, g))
-    th.save(out, path)
+    _save(out, "transforms")
     print("transforms.pt:", list(out), "runs case:", nw.tolist(), ew.tolist())
 
 
@@ -152,14 +164,13 @@ def gen_counting():
                         outputs={k: (v.detach().clone() if isinstance(v, th.Tensor) else None) for k, v in o.items()},
                         loss=loss.detach().clone(), grads=_grads(model))
     out["_batch"] = dict(pattern=_np(pd_), graph=_np(gd_), counts=counts, cfg=cfg, model_cfg=mc)
-    th.save(out, os.path.join(OUT, "counting_models.pt"))
+    _save(out, "counting_models")
     print("counting_models.pt:", [k for k in out if not k.startswith("_")])
 
 
 def gen_counting_rgcn():
     """SURVEY.md 8(f) rank 1: the reference's RGCN class, added to counting_models.pt (same batch as gen_counting)."""
-    path = os.path.join(OUT, "counting_models.pt")
-    out = th.load(path, weights_only=False)
+    out = _load("counting_models")
     b = out["_batch"]
     pd_, gd_, counts, mc = b["pattern"], b["graph"], b["counts"], b["model_cfg"]
     variants = {
@@ -187,14 +198,13 @@ def gen_counting_rgcn():
         out[tag] = dict(name="RGCN", kwargs=kw, state_dict={k: v.clone() for k, v in model.state_dict().items()},
                         outputs={k: (v.detach().clone() if isinstance(v, th.Tensor) else None) for k, v in o.items()},
                         loss=loss.detach().clone(), grads=_grads(model))
-    th.save(out, path)
+    _save(out, "counting_models")
     print("counting_models.pt:", [k for k in out if not k.startswith("_")])
 
 
 def gen_counting_compgcn():
     """SURVEY.md 8(f) rank 1: the reference's CompGCN class, added to counting_models.pt (same batch as gen_counting)."""
-    path = os.path.join(OUT, "counting_models.pt")
-    out = th.load(path, weights_only=False)
+    out = _load("counting_models")
     b = out["_batch"]
     pd_, gd_, counts, mc = b["pattern"], b["graph"], b["counts"], b["model_cfg"]
     variants = {
@@ -222,14 +232,14 @@ def gen_counting_compgcn():
         out[tag] = dict(name="CompGCN", kwargs=kw, state_dict={k: v.clone() for k, v in model.state_dict().items()},
                         outputs={k: (v.detach().clone() if isinstance(v, th.Tensor) else None) for k, v in o.items()},
                         loss=loss.detach().clone(), grads=_grads(model))
-    th.save(out, path)
+    _save(out, "counting_models")
     print("counting_models.pt:", [k for k in out if not k.startswith("_")])
 
 
 def gen_counting_loss():
     """SURVEY.md 8(a21): the full back-propagated loss incl. match terms, produced by the reference's OWN train_epoch
     (train.py:596-1000, executed verbatim on one mini-batch) for the three criteria -> counting_loss.pt."""
-    base = th.load(os.path.join(OUT, "counting_models.pt"), weights_only=False)
+    base = _load("counting_models")
     b = base["_batch"]
     Lg = int(np.diff(b["graph"]["node_ptr"]).max())
     Le = int(np.diff(b["graph"]["edge_ptr"]).max())

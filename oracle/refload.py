@@ -1,9 +1,8 @@
-"""Import the UNMODIFIED reference sources from /root/reference under the shims.
+"""Import the UNMODIFIED reference sources from the checkout DN4GL_REFERENCE_ROOT names, under the shims.
 
-TEST SCAFFOLDING.  Works only in the build container (the GPU box has no /root/reference);
-everything that needs it is guarded by ``available()``.  Used by ``oracle/gen_golden.py``
-to produce tests/golden/* and by the ``reference-live`` CPU tests that re-check the
-standalone restatement (oracle/transforms.py, oracle/models.py) against the reference.
+TEST SCAFFOLDING.  Works only where such a checkout exists; everything that needs it is guarded by
+``available()``.  Used by ``oracle/gen_golden.py`` to produce tests/golden/* and by the ``reference-live`` CPU tests
+that re-check the standalone restatement (oracle/transforms.py, oracle/models.py) against the reference.
 """
 import ast
 import collections.abc
@@ -15,7 +14,7 @@ import types
 
 import numpy as np
 
-REF_ROOT = os.environ.get("DN4GL_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("DN4GL_REFERENCE_ROOT") or ""
 _SUB = os.path.join(REF_ROOT, "subgraph_isomorphism")
 _CLS = os.path.join(REF_ROOT, "graph_classification")
 

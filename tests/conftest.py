@@ -10,20 +10,20 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box via gpurun)")
-    config.addinivalue_line("markers", "reference_live: executes the unmodified reference from /root/reference "
-                                       "(build container only; skipped elsewhere)")
+    config.addinivalue_line("markers", "reference_live: executes the unmodified original project from the checkout "
+                                       "DN4GL_REFERENCE_ROOT names (skipped without one)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    ref = os.path.isdir(os.environ.get("DN4GL_REFERENCE_ROOT", "/root/reference"))
+    ref = os.path.isdir(os.environ.get("DN4GL_REFERENCE_ROOT") or "")
     for it in items:
         if "gpu" in it.keywords and not has_gpu:
             it.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "reference_live" in it.keywords and not ref:
-            it.add_marker(pytest.mark.skip(reason="/root/reference not present"))
+            it.add_marker(pytest.mark.skip(reason="DN4GL_REFERENCE_ROOT names no checkout of the original project"))
 
 
 @pytest.fixture(scope="session")

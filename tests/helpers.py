@@ -8,7 +8,13 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_golden(name):
-    return torch.load(os.path.join(GOLDEN, name), weights_only=False)
+    """a .pt file, or a directory holding one .pt file per key (the larger sets, split to keep every file small):
+    {key: value} with the key being the file's path under the directory without ".pt"."""
+    path = os.path.join(GOLDEN, name)
+    if not os.path.isdir(path):
+        return torch.load(path, weights_only=False)
+    return {os.path.relpath(os.path.join(d, f), path)[:-3]: torch.load(os.path.join(d, f), weights_only=False)
+            for d, _, files in os.walk(path) for f in files if f.endswith(".pt")}
 
 
 from oracle.models import counting_cfg_from_kwargs as oracle_cfg  # noqa: E402,F401  (kept under its old name for the tests)

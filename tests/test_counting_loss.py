@@ -26,7 +26,7 @@ def golden_grads_by_name(sd, names, shared):
 
 @pytest.mark.parametrize("tag", CASES)
 def test_bp_loss_matches_reference_train_epoch_golden(tag):
-    gold, base = load_golden("counting_loss.pt"), load_golden("counting_models.pt")
+    gold, base = load_golden("counting_loss.pt"), load_golden("counting_models")
     g, b = gold[tag], base["_batch"]
     m, c = base[g["model"]], g["conf"]
     sd = {k: v.clone().requires_grad_(v.is_floating_point()) for k, v in g["state_dict"].items()}

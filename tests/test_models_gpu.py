@@ -55,7 +55,7 @@ def _check_outputs(out, ref):
                                  "CompGCN/mult_in_bn_unshared", "CompGCN/corr_out"])
 def test_counting_models_match_reference_golden(device, tag):
     from dummynode4graphlearning_b200.graph import BatchedGraph
-    gold = load_golden("counting_models.pt")
+    gold = load_golden("counting_models")
     g, b = gold[tag], gold["_batch"]
     model = _counting_model(g["name"], g["kwargs"], g["state_dict"], device)
     pattern = BatchedGraph.from_batch(b["pattern"], device)

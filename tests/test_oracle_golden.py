@@ -15,9 +15,20 @@ CONJ_KEYS = ("node_ptr", "edge_ptr", "src", "dst", "vid", "vlabel", "v_is_dummy"
              "e_is_dummy")
 
 
+@pytest.fixture(scope="module", autouse=True)
+def golden_thread_count():
+    """the fp32 goldens carry the reduction order of torch's CPU kernels split over at least 8 intra-op threads (the split
+    stops changing there at these sizes); on fewer threads the oracle rounds differently by a few 1e-6, more than the
+    1e-6 bars below allow"""
+    before = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(before)
+
+
 @pytest.fixture(scope="module")
 def gold_t():
-    return load_golden("transforms.pt")
+    return load_golden("transforms")
 
 
 @pytest.mark.parametrize("case", ["appB", "mutag12", "proteins8"])
@@ -139,7 +150,7 @@ def test_closed_forms_on_random_graphs():
                                  "RGCN/none_basis4_bn_unshared", "CompGCN/mult_none", "CompGCN/sub_both_node_edge",
                                  "CompGCN/mult_in_bn_unshared", "CompGCN/corr_out"])
 def test_counting_oracle_matches_reference_golden(tag):
-    gold = load_golden("counting_models.pt")
+    gold = load_golden("counting_models")
     g, b = gold[tag], gold["_batch"]
     sd = {k: v.clone().requires_grad_(v.is_floating_point()) for k, v in g["state_dict"].items()}
     out = OM.counting_model(sd, b["pattern"], b["graph"], oracle_cfg(g["name"], g["kwargs"]))
@@ -156,7 +167,11 @@ def test_counting_oracle_matches_reference_golden(tag):
     loss = OM.counting_loss(out, torch.from_numpy(b["counts"]), rep_reg_w=1e-3)
     assert_close_rel(loss, g["loss"], 1e-6, "loss")
     loss.backward()
-    # shared modules appear under both prefixes in the state_dict; named_parameters() dedupes to the first name
+    # shared modules appear under both prefixes in the state_dict; named_parameters() dedupes to the first name.
+    # A bias that feeds a BatchNorm has a mathematically zero gradient: only rounding noise is left on both sides (it
+    # changes with the BLAS code path of the host), compared against an absolute floor tied to the largest gradient
+    gmax = max(float(r.abs().max()) for r in g["grads"].values() if r is not None)
+    batch_norm = any(v for k, v in g["kwargs"].items() if k.endswith("_batch_norm"))
     for n, ref in g["grads"].items():
         got = sd[n].grad
         alias = n.replace("g_rep_net", "p_rep_net", 1) if n.startswith("g_rep_net") else None
@@ -164,7 +179,8 @@ def test_counting_oracle_matches_reference_golden(tag):
             got = got + sd[alias].grad if got is not None else sd[alias].grad
         if ref is None:   # frozen encoder tables / EquivariantEmbedding.row_vec never get a gradient (App. A-13)
             continue
-        assert_close_rel(got, ref, 1e-5, "grad " + n)
+        pre_bn_bias = n.endswith(".bias") and batch_norm and float(ref.abs().max()) <= 1e-6 * gmax
+        assert_close_rel(got, ref, 1e-5, "grad " + n, atol=1e-6 * gmax if pre_bn_bias else 0.0)
 
 
 @pytest.mark.parametrize("tag", ["GIN/mutag_dummy", "GIN/mutag_conj_eps", "RGIN/mutag_dummy"])

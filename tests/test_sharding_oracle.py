@@ -38,7 +38,7 @@ def take(b, idx):
 
 @pytest.mark.parametrize("tag", ["RGIN/bdd4", "DMPNN/node_edge"])
 def test_shard_padded_to_batch_wide_lengths_reproduces_full_batch(tag):
-    gold = load_golden("counting_models.pt")
+    gold = load_golden("counting_models")
     g, b = gold[tag], gold["_batch"]
     torch.manual_seed(0)
     sd = {k: v.clone() for k, v in g["state_dict"].items()}

@@ -263,7 +263,7 @@ def test_augmentation_flags_match_golden_and_oracle(device, shape):
     from dummynode4graphlearning_b200.graph import BatchedGraph
     from helpers import batches_equal, load_golden
 
-    g = load_golden("transforms.pt")["aug/" + shape]
+    g = load_golden("transforms")["aug/" + shape]
     cfg = g["cfg"]
     E_KEYS = ("edge_ptr", "src", "dst", "eid", "elabel")
     SUB_KEYS = ("node_ptr", "edge_ptr", "src", "dst", "vid", "vlabel", "v_is_dummy", "eid", "elabel", "e_is_dummy", "e_is_reversed")
@@ -322,7 +322,7 @@ def test_match_weights_golden(device, case):
     from dummynode4graphlearning_b200 import transforms as T
     from dummynode4graphlearning_b200.subgraph_isomorphism import matching as M
     from helpers import load_golden
-    g = load_golden("transforms.pt")["match/" + case]
+    g = load_golden("transforms")["match/" + case]
     sub = M.pack_subisomorphisms(g["mats"], device)
     pb, gb = T.to_device(g["pattern"], device), T.to_device(g["graph"], device)
     assert np.array_equal(M.node_weights(sub, gb).cpu().numpy(), g["node_weights"])

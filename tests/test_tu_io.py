@@ -13,7 +13,7 @@ from oracle import transforms as OT
 @pytest.mark.parametrize("case", ["appB", "mutag12", "proteins8"])
 def test_writer_matches_reference_save_graph_data(case):
     """tu_file_lines(CONJ batch) == the text the reference's save_graph_data wrote for the same graphs."""
-    g = load_golden("transforms.pt")["tu/" + case]
+    g = load_golden("transforms")["tu/" + case]
     conj = OT.tu_conjugate(OT.tu_add_dummy(g["inp"]))
     mine = tuio.tu_file_lines(conj)
     for suffix, lines in g["conj_files"].items():
@@ -24,7 +24,7 @@ def test_writer_matches_reference_save_graph_data(case):
 def test_reader_round_trip_and_reference_loader_equivalence(case):
     """write (reference layout) -> load_tu_dir -> the same batch; and dummy-augmenting the loaded batch gives what the
     reference's load_graph_data_from_TUDatadir(with_dummy=True) built from those files (golden)."""
-    g = load_golden("transforms.pt")["tu/" + case]
+    g = load_golden("transforms")["tu/" + case]
     b = dict(g["inp"])
     b["vid"] = np.concatenate([np.arange(n) for n in np.diff(b["node_ptr"])]).astype(np.int32)
     b["eid"] = np.concatenate([np.arange(n) for n in np.diff(b["edge_ptr"])]).astype(np.int32)

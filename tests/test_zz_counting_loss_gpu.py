@@ -26,7 +26,7 @@ def _model(name, kw, sd, device):
 def test_full_bp_loss_matches_reference_train_epoch_golden(device, tag):
     from dummynode4graphlearning_b200.graph import BatchedGraph
     from dummynode4graphlearning_b200.subgraph_isomorphism.losses import counting_bp_loss
-    gold, base = load_golden("counting_loss.pt"), load_golden("counting_models.pt")
+    gold, base = load_golden("counting_loss.pt"), load_golden("counting_models")
     g, b = gold[tag], base["_batch"]
     m, c = base[g["model"]], g["conf"]
     model = _model(m["name"], m["kwargs"], g["state_dict"], device)

@@ -66,8 +66,6 @@ class _Lib:
         if self._dll.dn4gl_version() != 1:
             raise Dn4glError("libdn4gl.so ABI version mismatch")
         self.launches = 0  # number of C-ABI compute calls issued (bench.py reports it)
-        if os.environ.get("DN4GL_SM_LIMIT"):
-            self._dll.dn4gl_set_sm_limit(int(os.environ["DN4GL_SM_LIMIT"]))
 
     def raw(self, name):
         return getattr(self._dll, name)

@@ -14,7 +14,6 @@ template <int LANES, int VEC>
 __global__ void __launch_bounds__(256)
 spmm_rows_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col, const float4 *__restrict__ x,
                  float4 *__restrict__ out, int64_t N, float self_scale, const float *__restrict__ eps_dev, int heavy_thr) {
-    DN_PDL_WAIT();
     if (eps_dev != nullptr) self_scale = 1.f + __ldg(eps_dev);
     constexpr int ROWS = 256 / LANES;
     constexpr int U = (VEC == 1) ? 8 : (VEC == 2 ? 4 : 2);
@@ -73,7 +72,6 @@ __global__ void __launch_bounds__(256)
 spmm_heavy_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict__ col, const float4 *__restrict__ x,
                   float4 *__restrict__ out, float self_scale, const float *__restrict__ eps_dev,
                   const int32_t *__restrict__ heavy_rows, const int32_t *__restrict__ heavy_count) {
-    DN_PDL_WAIT();
     if (eps_dev != nullptr) self_scale = 1.f + __ldg(eps_dev);
     constexpr int SUBS = 256 / LANES;
     constexpr int DV = LANES * VEC;
@@ -139,11 +137,11 @@ static int launch_spmm(const int32_t *row_ptr, const int32_t *col, const float *
                        int heavy_thr, cudaStream_t st) {
     constexpr int ROWS = 256 / LANES;
     const bool heavy = heavy_rows != nullptr && heavy_count != nullptr && heavy_thr > 0;
-    DN_LAUNCH((spmm_rows_kernel<LANES, VEC>), static_cast<unsigned>(ceil_div64(N, ROWS)), 256, 0, st,
+    spmm_rows_kernel<LANES, VEC><<<static_cast<unsigned>(ceil_div64(N, ROWS)), 256, 0, st>>>(
         row_ptr, col, reinterpret_cast<const float4 *>(x), reinterpret_cast<float4 *>(out), N, self_scale, eps_dev,
         heavy ? heavy_thr : 0);
     if (heavy) {
-        DN_LAUNCH((spmm_heavy_kernel<LANES, VEC>), dn4gl_num_sms() * 4, 256, 0, st,
+        spmm_heavy_kernel<LANES, VEC><<<dn4gl_num_sms() * 4, 256, 0, st>>>(
             row_ptr, col, reinterpret_cast<const float4 *>(x), reinterpret_cast<float4 *>(out), self_scale, eps_dev,
             heavy_rows, heavy_count);
     }
@@ -186,7 +184,6 @@ template <int LANES, int VEC>
 __global__ void __launch_bounds__(256)
 segment_sum_kernel(const int32_t *__restrict__ seg_ptr, const uint8_t *__restrict__ mask,
                    const float4 *__restrict__ x, float4 *__restrict__ out, int B, int mode) {
-    DN_PDL_WAIT();
     constexpr int SUBS = 256 / LANES;
     constexpr int DV = LANES * VEC;
     __shared__ float4 part[256 * VEC];
@@ -235,7 +232,6 @@ segment_sum_kernel(const int32_t *__restrict__ seg_ptr, const uint8_t *__restric
 __global__ void __launch_bounds__(256)
 segment_sum_generic(const int32_t *__restrict__ seg_ptr, const uint8_t *__restrict__ mask,
                     const float *__restrict__ x, float *__restrict__ out, int B, int D, int mode) {
-    DN_PDL_WAIT();
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= B) return;
     const int beg = seg_ptr[warp], end = seg_ptr[warp + 1];
@@ -254,7 +250,6 @@ template <int DMAX>
 __global__ void __launch_bounds__(256)
 segment_sum_narrow(const int32_t *__restrict__ seg_ptr, const uint8_t *__restrict__ mask, const float *__restrict__ x,
                    float *__restrict__ out, int B, int D, int mode) {
-    DN_PDL_WAIT();
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= B) return;
     const int beg = seg_ptr[warp], end = seg_ptr[warp + 1];
@@ -289,7 +284,7 @@ extern "C" int dn4gl_segment_sum_f32(const int32_t *seg_ptr, const uint8_t *mask
     const bool vec_ok = (D % 4 == 0) && aligned16(x) && aligned16(out);
     const int dv = vec_ok ? D / 4 : 0;
 #define SEG_CASE(L, V)                                                                                       \
-    DN_LAUNCH((segment_sum_kernel<L, V>), grid, 256, 0, st, seg_ptr, mask, reinterpret_cast<const float4 *>(x),       \
+    segment_sum_kernel<L, V><<<grid, 256, 0, st>>>(seg_ptr, mask, reinterpret_cast<const float4 *>(x),       \
                                                    reinterpret_cast<float4 *>(out), B, mode);                \
     break
     switch (dv) {
@@ -300,10 +295,10 @@ extern "C" int dn4gl_segment_sum_f32(const int32_t *seg_ptr, const uint8_t *mask
         case 128: SEG_CASE(32, 4);
         default:
             if (D <= 8)
-                DN_LAUNCH(segment_sum_narrow<8>, static_cast<unsigned>(ceil_div64(static_cast<int64_t>(B) * 32, 256)), 256, 0, st,
+                segment_sum_narrow<8><<<static_cast<unsigned>(ceil_div64(static_cast<int64_t>(B) * 32, 256)), 256, 0, st>>>(
                     seg_ptr, mask, x, out, B, D, mode);
             else
-                DN_LAUNCH(segment_sum_generic, static_cast<unsigned>(ceil_div64(static_cast<int64_t>(B) * 32, 256)), 256, 0, st,
+                segment_sum_generic<<<static_cast<unsigned>(ceil_div64(static_cast<int64_t>(B) * 32, 256)), 256, 0, st>>>(
                     seg_ptr, mask, x, out, B, D, mode);
     }
 #undef SEG_CASE
@@ -314,7 +309,6 @@ extern "C" int dn4gl_segment_sum_f32(const int32_t *seg_ptr, const uint8_t *mask
 __global__ void segment_bcast_kernel(const int32_t *__restrict__ seg_ptr, const uint8_t *__restrict__ mask,
                                      const float *__restrict__ g, float *__restrict__ gx, int B, int64_t N, int D,
                                      int mode) {
-    DN_PDL_WAIT();
     int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= N * D) return;
     int64_t v = i / D;
@@ -331,7 +325,7 @@ extern "C" int dn4gl_segment_bcast_f32(const int32_t *seg_ptr, const uint8_t *ma
     DN_ARG(B >= 0 && N >= 0 && D > 0 && (mode == 0 || mode == 1));
     if (N == 0) return DN4GL_OK;
     DN_ARG(seg_ptr && g && gx);
-    DN_LAUNCH(segment_bcast_kernel, static_cast<unsigned>(ceil_div64(N * D, 256)), 256, 0, as_stream(stream),
+    segment_bcast_kernel<<<static_cast<unsigned>(ceil_div64(N * D, 256)), 256, 0, as_stream(stream)>>>(
         seg_ptr, mask, g, gx, B, N, D, mode);
     DN_LAUNCHED();
     return DN4GL_OK;
@@ -341,7 +335,6 @@ extern "C" int dn4gl_segment_bcast_f32(const int32_t *seg_ptr, const uint8_t *ma
 // left-padded batchify (utils/dl.py:51-81 with pre_pad=True) and its adjoint.
 __global__ void pad_segments_kernel(const int32_t *__restrict__ seg_ptr, const uint8_t *__restrict__ mask,
                                     const float *__restrict__ x, float *__restrict__ out, int B, int Lmax, int D) {
-    DN_PDL_WAIT();
     int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     int64_t total = static_cast<int64_t>(B) * Lmax * D;
     if (i >= total) return;
@@ -362,7 +355,6 @@ __global__ void pad_segments_kernel(const int32_t *__restrict__ seg_ptr, const u
 __global__ void unpad_segments_kernel(const int32_t *__restrict__ seg_ptr, const uint8_t *__restrict__ mask,
                                       const float *__restrict__ g, float *__restrict__ gx, int B, int Lmax, int D,
                                       int64_t N) {
-    DN_PDL_WAIT();
     int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= N * D) return;
     int64_t r = i / D;
@@ -380,8 +372,8 @@ extern "C" int dn4gl_pad_segments_f32(const int32_t *seg_ptr, const uint8_t *mas
     int64_t total = static_cast<int64_t>(B) * Lmax * D;
     if (total == 0) return DN4GL_OK;
     DN_ARG(seg_ptr && x && out);
-    DN_LAUNCH(pad_segments_kernel, static_cast<unsigned>(ceil_div64(total, 256)), 256, 0, as_stream(stream), seg_ptr, mask, x,
-                                                                                                       out, B, Lmax, D);
+    pad_segments_kernel<<<static_cast<unsigned>(ceil_div64(total, 256)), 256, 0, as_stream(stream)>>>(seg_ptr, mask, x,
+                                                                                                      out, B, Lmax, D);
     DN_LAUNCHED();
     return DN4GL_OK;
 }
@@ -391,7 +383,7 @@ extern "C" int dn4gl_unpad_segments_f32(const int32_t *seg_ptr, const uint8_t *m
     DN_ARG(B >= 0 && Lmax >= 0 && D > 0 && N >= 0);
     if (N == 0) return DN4GL_OK;
     DN_ARG(seg_ptr && g && gx);
-    DN_LAUNCH(unpad_segments_kernel, static_cast<unsigned>(ceil_div64(N * D, 256)), 256, 0, as_stream(stream),
+    unpad_segments_kernel<<<static_cast<unsigned>(ceil_div64(N * D, 256)), 256, 0, as_stream(stream)>>>(
         seg_ptr, mask, g, gx, B, Lmax, D, N);
     DN_LAUNCHED();
     return DN4GL_OK;
@@ -402,7 +394,6 @@ extern "C" int dn4gl_unpad_segments_f32(const int32_t *seg_ptr, const uint8_t *m
 __global__ void label_filter_kernel(const int32_t *__restrict__ g_ptr, const int32_t *__restrict__ g_label,
                                     const int32_t *__restrict__ p_ptr, const int32_t *__restrict__ p_label, int B,
                                     int Lp_max, float *__restrict__ gate, int64_t Ng) {
-    DN_PDL_WAIT();
     int64_t v = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (v >= Ng) return;
     int b = segment_of(g_ptr, B, v);
@@ -419,7 +410,7 @@ extern "C" int dn4gl_label_filter_gate(const int32_t *g_ptr, const int32_t *g_la
     DN_ARG(B >= 0 && Ng >= 0);
     if (Ng == 0) return DN4GL_OK;
     DN_ARG(g_ptr && g_label && p_ptr && p_label && gate);
-    DN_LAUNCH(label_filter_kernel, static_cast<unsigned>(ceil_div64(Ng, 256)), 256, 0, as_stream(stream),
+    label_filter_kernel<<<static_cast<unsigned>(ceil_div64(Ng, 256)), 256, 0, as_stream(stream)>>>(
         g_ptr, g_label, p_ptr, p_label, B, Lp_max, gate, Ng);
     DN_LAUNCHED();
     return DN4GL_OK;
@@ -432,7 +423,6 @@ extern "C" int dn4gl_label_filter_gate(const int32_t *g_ptr, const int32_t *g_la
 // for the gradient  g_logp[b, c] = (c == y_b) ? -g / B : 0.
 __global__ void __launch_bounds__(1024) nll_mean_fwd_kernel(const float *__restrict__ logp, const int64_t *__restrict__ y,
                                                            int B, int C, float *__restrict__ loss) {
-    DN_PDL_WAIT();
     __shared__ float red[1024];
     float s = 0.f;
     for (int b = threadIdx.x; b < B; b += 1024) {
@@ -450,7 +440,6 @@ __global__ void __launch_bounds__(1024) nll_mean_fwd_kernel(const float *__restr
 
 __global__ void nll_mean_bwd_kernel(const float *__restrict__ g, const int64_t *__restrict__ y, int B, int C,
                                     float *__restrict__ g_logp) {
-    DN_PDL_WAIT();
     const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= static_cast<int64_t>(B) * C) return;
     const int b = static_cast<int>(i / C), c = static_cast<int>(i - static_cast<int64_t>(b) * C);
@@ -459,7 +448,7 @@ __global__ void nll_mean_bwd_kernel(const float *__restrict__ g, const int64_t *
 
 extern "C" int dn4gl_nll_mean_f32(const float *logp, const int64_t *y, int32_t B, int32_t C, float *loss, void *stream) {
     DN_ARG(B >= 0 && C > 0 && loss != nullptr && (B == 0 || (logp != nullptr && y != nullptr)));
-    DN_LAUNCH(nll_mean_fwd_kernel, 1, 1024, 0, as_stream(stream), logp, y, B, C, loss);
+    nll_mean_fwd_kernel<<<1, 1024, 0, as_stream(stream)>>>(logp, y, B, C, loss);
     DN_LAUNCHED();
     return DN4GL_OK;
 }
@@ -468,7 +457,7 @@ extern "C" int dn4gl_nll_mean_bwd_f32(const float *g, const int64_t *y, int32_t 
     DN_ARG(B >= 0 && C > 0);
     if (B == 0) return DN4GL_OK;
     DN_ARG(g != nullptr && y != nullptr && g_logp != nullptr);
-    DN_LAUNCH(nll_mean_bwd_kernel, static_cast<unsigned>(ceil_div64(static_cast<int64_t>(B) * C, 256)), 256, 0, as_stream(stream),
+    nll_mean_bwd_kernel<<<static_cast<unsigned>(ceil_div64(static_cast<int64_t>(B) * C, 256)), 256, 0, as_stream(stream)>>>(
         g, y, B, C, g_logp);
     DN_LAUNCHED();
     return DN4GL_OK;
@@ -495,7 +484,6 @@ struct JkHeadPtrs {
 // one warp per graph; lane c ends up with score[b, c] (C <= 32)
 __global__ void __launch_bounds__(256) jk_head_fwd_kernel(JkHeadPtrs p, int L, int B, int D, int C,
                                                          const int32_t *__restrict__ seg_ptr, float *__restrict__ logp) {
-    DN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
     if (b >= B) return;
@@ -535,7 +523,6 @@ __global__ void __launch_bounds__(256) jk_head_bwd_kernel(JkHeadPtrs p, int L, i
                                                          const int32_t *__restrict__ seg_ptr, const float *__restrict__ g_logp,
                                                          const float *__restrict__ logp, float *__restrict__ part,
                                                          int *counter) {
-    DN_PDL_WAIT();
     extern __shared__ float jk_smem[];
     __shared__ int is_last;
     const int LD = L * D, NW = C * LD, NACC = NW + 2 * C;      // acc: dW (l, c, d) | sum_b gs[b, c] | sum_b n_b gs[b, c]
@@ -639,7 +626,7 @@ extern "C" int dn4gl_jk_head_fwd_f32(const float *const *pooled, const float *co
     if (B == 0) return DN4GL_OK;
     JkHeadPtrs p = {};
     DN_ARG(jk_fill(p, L, pooled, W, bias) && logp != nullptr);
-    DN_LAUNCH(jk_head_fwd_kernel, (B + 7) / 8, 256, 0, as_stream(stream), p, L, B, D, C, seg_ptr, logp);
+    jk_head_fwd_kernel<<<(B + 7) / 8, 256, 0, as_stream(stream)>>>(p, L, B, D, C, seg_ptr, logp);
     DN_LAUNCHED();
     return DN4GL_OK;
 }
@@ -657,8 +644,8 @@ extern "C" int dn4gl_jk_head_bwd_f32(const float *g_logp, const float *logp, con
         DN_ARG(pooled[l] && W[l] && g_pooled[l] && dW[l] && db[l]);
         p.pooled[l] = pooled[l]; p.W[l] = W[l]; p.g_pooled[l] = g_pooled[l]; p.dW[l] = dW[l]; p.db[l] = db[l];
     }
-    DN_LAUNCH(jk_head_bwd_kernel, jk_grid(B), 256, smem, as_stream(stream), p, L, B, D, C, seg_ptr, g_logp, logp,
-              static_cast<float *>(ws), counter);
+    jk_head_bwd_kernel<<<jk_grid(B), 256, smem, as_stream(stream)>>>(p, L, B, D, C, seg_ptr, g_logp, logp,
+                                                                     static_cast<float *>(ws), counter);
     DN_LAUNCHED();
     return DN4GL_OK;
 }

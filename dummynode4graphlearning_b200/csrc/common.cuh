@@ -40,46 +40,6 @@ void dn4gl_note_launches(int n);
     } while (0)
 #define DN_LAUNCHED() DN_LAUNCHED_N(1)
 
-// Programmatic dependent launch -- EXPERIMENT, compiled only with -DDN4GL_PDL (make libdn4gl_exp.so EXP_FLAGS=-DDN4GL_PDL);
-// the product build expands DN_LAUNCH to the plain <<<>>> launch and DN_PDL_WAIT to nothing (SASS unchanged).
-// With it, a kernel launched through DN_LAUNCH may become resident while its predecessor on the stream drains: its
-// on-chip prologue (shared-memory carve-up, mbarrier init, tensor-memory allocation) overlaps the predecessor's tail and
-// the launch latency disappears from the chain of ~110 small kernels a train step replays.  Contract: EVERY kernel
-// launched through DN_LAUNCH executes DN_PDL_WAIT() before its first global-memory access (reads AND writes: the
-// predecessor may still be reading what this kernel overwrites); the wait returns once all prerequisite grids have
-// completed and flushed, so ordering and results are those of the serial launch.
-// -DDN4GL_PDL (= 1): dependents are released as the predecessor's CTAs exit (implicit trigger).  -DDN4GL_PDL=2: every
-// kernel also releases ITS dependents right before it starts waiting, so the next kernel's CTAs become resident as soon
-// as all of this kernel's CTAs have been scheduled and an SM has room (they cannot displace CTAs of a running grid: the
-// release needs every CTA of the releasing grid to have started), and sit in their own wait until the chain reaches them.
-#ifdef DN4GL_PDL
-#if DN4GL_PDL >= 2
-#define DN_PDL_WAIT() asm volatile("griddepcontrol.launch_dependents;\n\tgriddepcontrol.wait;" ::: "memory")
-#else
-#define DN_PDL_WAIT() asm volatile("griddepcontrol.wait;" ::: "memory")
-#endif
-#ifdef __CUDACC__
-template <typename... P, typename... A>
-static inline void dn_launch_pdl(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, A &&...args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<P>(args)...);   // a failure is picked up by DN_LAUNCHED()
-}
-#endif
-#define DN_LAUNCH(kernel, grid, block, smem, stream, ...) dn_launch_pdl(kernel, grid, block, smem, stream, __VA_ARGS__)
-#else
-#define DN_PDL_WAIT()
-#define DN_LAUNCH(kernel, grid, block, smem, stream, ...) kernel<<<grid, block, smem, stream>>>(__VA_ARGS__)
-#endif
-
 static inline cudaStream_t as_stream(void *s) { return reinterpret_cast<cudaStream_t>(s); }
 static inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

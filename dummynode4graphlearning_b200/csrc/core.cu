@@ -28,8 +28,6 @@ extern "C" int dn4gl_set_device(int device) {
     return DN4GL_OK;
 }
 
-static int g_sm_limit = 0;   // 0 = all SMs of the device
-
 int dn4gl_num_sms() {
     static int cached = 0;
     if (cached == 0) {
@@ -40,17 +38,7 @@ int dn4gl_num_sms() {
         else
             cached = 148;
     }
-    return (g_sm_limit > 0 && g_sm_limit < cached) ? g_sm_limit : cached;
-}
-
-// Process-wide cap on the SM count the library sizes its grids with (persistent kernels launch one CTA, or a fixed
-// number of CTAs, per SM).  A pipeline that runs the graph transforms on a second stream next to the train step leaves a
-// few SMs to that stream this way: the train step's persistent kernels own every register of the SMs they run on, so the
-// transform's chain of ~60 small kernels would otherwise wait for a whole train kernel (15-50 us) at every link.
-extern "C" int dn4gl_set_sm_limit(int n) {
-    DN_ARG(n >= 0);
-    g_sm_limit = n;
-    return DN4GL_OK;
+    return cached;
 }
 
 // -------------------------------------------------------------------------------------------

@@ -21,7 +21,6 @@ constexpr int ATB_MAX_TILES = 256;  // (Ka/4) * (Kb/4) register tiles of 4 x 4 m
 __global__ void __launch_bounds__(ATB_THREADS)
 atb_partial_kernel(const float *__restrict__ A, const float *__restrict__ B, int64_t N, int Ka, int Kb, int GA, int GB,
                    int64_t rows_per_cta, float *__restrict__ partial /* [grid][Ka*Kb + Ka] */) {
-    DN_PDL_WAIT();
     extern __shared__ __align__(16) float smem[];
     const int PA = 4 * GA, PB = 4 * GB;
     float *sA = smem;                      // [ATB_ROWS][PA]
@@ -118,7 +117,6 @@ atb_partial_kernel(const float *__restrict__ A, const float *__restrict__ B, int
 __global__ void __launch_bounds__(256)
 atb_reduce_kernel(const float *__restrict__ partial, int P, int KaKb, int Ka, float *__restrict__ C,
                   float *__restrict__ colsum) {
-    DN_PDL_WAIT();
     __shared__ float red[8][33];
     const int o = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int i = blockIdx.x * 32 + o;
@@ -180,9 +178,9 @@ extern "C" int dn4gl_atb_f32(const float *A, const float *B, float *C, float *co
     size_t smem = sizeof(float) * static_cast<size_t>(ATB_ROWS) * 4 * (GA + GB);
     const size_t red = sizeof(float) * static_cast<size_t>(RS) * GA * GB * 20;
     if (red > smem) smem = red;
-    DN_LAUNCH(atb_partial_kernel, grid, ATB_THREADS, smem, st, A, B, N, Ka, Kb, GA, GB, rows_per_cta, partial);
+    atb_partial_kernel<<<grid, ATB_THREADS, smem, st>>>(A, B, N, Ka, Kb, GA, GB, rows_per_cta, partial);
     const int total = Ka * Kb + Ka;
-    DN_LAUNCH(atb_reduce_kernel, (total + 31) / 32, 256, 0, st, partial, grid, Ka * Kb, Ka, C, colsum_A);
+    atb_reduce_kernel<<<(total + 31) / 32, 256, 0, st>>>(partial, grid, Ka * Kb, Ka, C, colsum_A);
     DN_LAUNCHED_N(2);
     return DN4GL_OK;
 }

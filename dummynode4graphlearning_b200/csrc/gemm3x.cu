@@ -63,7 +63,6 @@ __device__ __forceinline__ void mbar_arrive_g(uint32_t bar) {
 template <int MT>
 __global__ void __launch_bounds__(256) gemm3x_prep_kernel(const float *__restrict__ B, int ldb, int layout, int K, int M, int kchunks,
                                                           float *__restrict__ Bp) {
-    DN_PDL_WAIT();
     const int kc = blockIdx.x, ct = blockIdx.y;
     char *blk = reinterpret_cast<char *>(Bp) + (static_cast<size_t>(ct) * kchunks + kc) * MT * 256;
     for (int idx = threadIdx.x; idx < MT * 8; idx += 256) {
@@ -106,7 +105,6 @@ struct GemmCfg {
 template <int MT>
 __global__ void __launch_bounds__(GemmCfg<MT>::NT, 1) gemm3x_kernel(const GemmArgs a) {
     using C = GemmCfg<MT>;
-    DN_PDL_WAIT();
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * C::STAGES + 4 + 2 * C::RS];
     __shared__ uint32_t tmem_ptr;
@@ -412,9 +410,9 @@ static int launch_gemm(const GemmArgs &a, const float *B, int ldb, int layout, f
             return -1;
         attr_done = true;
     }
-    DN_LAUNCH((gemm3x_prep_kernel<MT>), dim3(a.kchunks, a.col_tiles), 256, 0, s, B, ldb, layout, a.K, a.M, a.kchunks, Bp);
+    gemm3x_prep_kernel<MT><<<dim3(a.kchunks, a.col_tiles), 256, 0, s>>>(B, ldb, layout, a.K, a.M, a.kchunks, Bp);
     const int tiles = a.row_tiles * a.col_tiles, sms = dn4gl_num_sms();
-    DN_LAUNCH((gemm3x_kernel<MT>), tiles < sms ? tiles : sms, C::NT, C::SMEM, s, a);
+    gemm3x_kernel<MT><<<tiles < sms ? tiles : sms, C::NT, C::SMEM, s>>>(a);
     return 0;
 }
 

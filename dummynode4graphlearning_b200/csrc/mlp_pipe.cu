@@ -21,7 +21,6 @@
 // measures: (1) all A_lo MMAs are issued FIRST (their sum is 2^-11 of the result, truncation at that magnitude is
 // harmless) and only then the A_hi MMAs; (2) the A_hi k-steps are spread over NACC accumulators that the epilogue
 // adds in round-to-nearest fp32.  The double-buffered accumulators hide the extra tensor-memory reads.
-#include <stdlib.h>
 #include <type_traits>
 #include "common.cuh"
 #include "tc_common.cuh"
@@ -207,7 +206,6 @@ lin_fwd_pipe_kernel(const LinFwdArgs a, const BnFinalArgs f, int *__restrict__ c
     }
     if (w == C::W_MMA) tc_alloc(s_u32(&tmem_ptr), C::TCOLS);
     __syncthreads();
-    DN_PDL_WAIT();   // (experiment) everything above is on-chip; global memory is first touched below
     // weights: W (M x K) row-major = K-major B operand, zero-padded to MP x KP, split once: per 32-float K panel the MP
     // hi rows then the MP lo rows, so that ONE MMA with N = 2 MP multiplies an A tile with [W_hi | W_lo]
     for (int i = t; i < MP * (KP / 4); i += C::NT) {
@@ -530,7 +528,7 @@ int launch_fwd_pipe(const LinFwdArgs &a, const BnFinalArgs &f, int *counter, cud
         if (launch_coop(lin_fwd_pipe_kernel<KP, MP, NACC, NBUF_A, RING, NCV, NEPI, NACCBUF>, grid, C::NT, C::SMEM, s, a, f, counter) != cudaSuccess)
             return -1;
     } else {
-        DN_LAUNCH((lin_fwd_pipe_kernel<KP, MP, NACC, NBUF_A, RING, NCV, NEPI, NACCBUF>), grid, C::NT, C::SMEM, s, a, f, counter);
+        lin_fwd_pipe_kernel<KP, MP, NACC, NBUF_A, RING, NCV, NEPI, NACCBUF><<<grid, C::NT, C::SMEM, s>>>(a, f, counter);
     }
     return grid;
 }
@@ -603,7 +601,6 @@ lin_bwd_pipe_kernel(const LinBwdArgs a, float *__restrict__ dW, float *__restric
     }
     if (w == C::W_MMA) tc_alloc(s_u32(&tmem_ptr), C::TCOLS);
     __syncthreads();
-    DN_PDL_WAIT();
     const bool want_gx = a.GX != nullptr, has_bn = a.bn != nullptr, has_bn_in = a.in_bn != nullptr, has_seg = a.Gseg != nullptr;
     // weights as they are stored: rows m (the data GEMM's K), k contiguous (its N) -> MN-major B operand, hi panels then lo
     if (want_gx) {
@@ -1066,7 +1063,5 @@ int dn4gl_pipe_lin_bwd(LinBwdArgs a, float *dW, float *db, float *sums_prev, voi
     const size_t P = static_cast<size_t>(bwd_pipe_part_floats(KP, MP));
     a.part = static_cast<float *>(ws);
     float *gpart = reinterpret_cast<float *>(static_cast<char *>(ws) + align_up(static_cast<size_t>(dn4gl_num_sms()) * P * sizeof(float), 256));
-    static const int nepi = getenv("DN4GL_BWD_NEPI") ? atoi(getenv("DN4GL_BWD_NEPI")) : 1;     // experiment switch
-    if (nepi == 2) return launch_bwd_pipe<32, 32, 3, 8, 2>(a, dW, db, sums_prev, gpart, counters, s);
     return launch_bwd_pipe<32, 32, 3, 8, 1>(a, dW, db, sums_prev, gpart, counters, s);
 }

@@ -21,7 +21,6 @@
 // (rows = K) by the weight-gradient GEMM.  One thread issues the MMAs; completion arrives on an mbarrier through
 // tcgen05.commit; accumulators come back with tcgen05.ld (32 lanes x 32 columns per warp) and leave through a staging
 // tile so that global stores are 128-bit and coalesced.  All reductions are fixed-order (no float atomics).
-#include <stdlib.h>
 #include "common.cuh"
 #include "tc_common.cuh"
 
@@ -70,7 +69,6 @@ __global__ void __launch_bounds__(NT) lin_fwd_kernel(const LinFwdArgs a) {
     }
     if (w == 0) tc_alloc(s_u32(&tmem_ptr), TCOLS);
     __syncthreads();
-    DN_PDL_WAIT();   // (experiment) everything above is on-chip; global memory is first touched below
     // raw ring: tile j of this CTA lives in slot j % RING
     auto issue = [&](int j) {
         const int64_t tile = static_cast<int64_t>(blockIdx.x) + static_cast<int64_t>(j) * gridDim.x;
@@ -267,7 +265,6 @@ __global__ void __launch_bounds__(NT) lin_bwd_kernel(const LinBwdArgs a) {
     }
     if (w == 0) tc_alloc(s_u32(&tmem_ptr), TCOLS);
     __syncthreads();
-    DN_PDL_WAIT();   // (experiment) everything above is on-chip; global memory is first touched below
     const bool want_gx = a.GX != nullptr, has_bn = a.bn != nullptr, has_bn_in = a.in_bn != nullptr;
     auto issue = [&](int j) {
         const int64_t tile = static_cast<int64_t>(blockIdx.x) + static_cast<int64_t>(j) * gridDim.x;
@@ -546,7 +543,6 @@ __device__ __forceinline__ double group_sum(double (*sm)[33], int lane, int g, d
 __global__ void __launch_bounds__(1024)
 lin_bwd_reduce_kernel(const float *__restrict__ part, int nparts, int MP, int KP, int M, int K,
                       float *__restrict__ dW, float *__restrict__ db, float *__restrict__ sums_prev) {
-    DN_PDL_WAIT();
     __shared__ double sm[32][33];
     __shared__ float *sm_dst[32];
     const int stride = bwd_part_floats(KP, MP);
@@ -587,7 +583,6 @@ __global__ void __launch_bounds__(1024)
 bn_finalize_kernel(const float4 *__restrict__ part, int nparts, int MP, int M, int64_t N,
                    const float *__restrict__ gamma, const float *__restrict__ beta, float eps, float momentum,
                    float *__restrict__ bn_out, float *__restrict__ run_mean, float *__restrict__ run_var, long long *nbt) {
-    DN_PDL_WAIT();
     __shared__ double sm[32][33];
     __shared__ double sm_kstar[32];
     const int lane = threadIdx.x & 31, g = threadIdx.x >> 5;
@@ -654,7 +649,6 @@ bn_finalize_kernel(const float4 *__restrict__ part, int nparts, int MP, int M, i
 // out = act(bn(Y))  (the activation a stage hands to a non-MLP consumer: aggregation, readout)
 __global__ void bn_act_kernel(const float *__restrict__ Y, int64_t N, int M, const float *__restrict__ bn, int act, float slope,
                               float *__restrict__ out) {
-    DN_PDL_WAIT();
     const int CH = (M + 3) / 4;
     const bool vec = (M % 4 == 0) && aligned16_dev(Y) && aligned16_dev(out);
     const int64_t total = N * CH;
@@ -676,7 +670,6 @@ template <int CHP>
 __global__ void __launch_bounds__(256) bn_act_pool_kernel(const float *__restrict__ Y, int M, const float *__restrict__ bn, int act,
                                                           float slope, float *__restrict__ out, const int32_t *__restrict__ seg_ptr,
                                                           int B, int mode, float *__restrict__ pooled) {
-    DN_PDL_WAIT();
     constexpr int RP = 256 / CHP;
     __shared__ float red[8][4 * CHP];
     const int t = threadIdx.x, w = t >> 5, lane = t & 31, c = t % CHP, r0 = t / CHP;
@@ -731,7 +724,6 @@ __global__ void __launch_bounds__(256) bn_act_pool_kernel(const float *__restric
 
 // row -> segment index for contiguous segments (the `batch` vector of a PyG batch, as int32)
 __global__ void segment_ids_kernel(const int32_t *__restrict__ seg_ptr, int B, int64_t N, int32_t *__restrict__ out) {
-    DN_PDL_WAIT();
     const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i < N) out[i] = segment_of(seg_ptr, B, i);
 }
@@ -744,7 +736,6 @@ __global__ void __launch_bounds__(256) bn_bwd_sums_kernel(const float *__restric
                                                           int64_t N, int M, const float *__restrict__ bn, int act, float slope,
                                                           float *__restrict__ part /* [grid][2*4*CHP] */, float *__restrict__ sums,
                                                           int *__restrict__ counters) {
-    DN_PDL_WAIT();
     constexpr int RP = 256 / CHP;
     __shared__ float red[8][8 * CHP];
     __shared__ double dred[256];
@@ -852,7 +843,6 @@ __global__ void __launch_bounds__(256) bn_bwd_sums_kernel(const float *__restric
 template <int CHP>
 __global__ void __launch_bounds__(256) bn_stats_partial_kernel(const float *__restrict__ Y, int64_t N, int M, int MP,
                                                                float4 *__restrict__ part /* [grid][MP] */) {
-    DN_PDL_WAIT();
     constexpr int RP = 256 / CHP;
     __shared__ float red[8][8 * CHP];
     const int t = threadIdx.x, w = t >> 5, lane = t & 31, c = t % CHP, r0 = t / CHP;
@@ -908,7 +898,6 @@ template <int CHP>
 __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const float *__restrict__ G, const float *__restrict__ Y, int64_t N, int M,
                                                            const float *__restrict__ bn, const float *__restrict__ sums, int act,
                                                            float slope, float *__restrict__ GX) {
-    DN_PDL_WAIT();
     constexpr int RP = 256 / CHP;
     const int t = threadIdx.x, c = t % CHP, r0 = t / CHP;
     if (4 * c >= M) return;
@@ -934,7 +923,6 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const float *__restri
 // fixed-order dot product: per-CTA partial (tree in shared memory), the last CTA adds the partials in index order
 __global__ void __launch_bounds__(256) dot_kernel(const float *__restrict__ a, const float *__restrict__ b, int64_t n,
                                                   float *__restrict__ out, float *__restrict__ part, int *counter) {
-    DN_PDL_WAIT();
     __shared__ float red[256];
     __shared__ int is_last;
     const int t = threadIdx.x;
@@ -1029,7 +1017,7 @@ int launch_fwd(const LinFwdArgs &a, int *grid_out, cudaStream_t s) {
     const size_t smem = fwd_smem(KP, MP, RING);
     const int grid = tc_grid(a.N, smem, (TC_SPLIT_ACC < KP / 16 ? TC_SPLIT_ACC : KP / 16) * 2 * MP, NT_FWD);
     DN_CUDA(cudaFuncSetAttribute(lin_fwd_kernel<KP, MP, RING, NT_FWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    DN_LAUNCH((lin_fwd_kernel<KP, MP, RING, NT_FWD>), grid, NT_FWD, smem, s, a);
+    lin_fwd_kernel<KP, MP, RING, NT_FWD><<<grid, NT_FWD, smem, s>>>(a);
     *grid_out = grid;
     return 0;
 }
@@ -1040,7 +1028,7 @@ int launch_bwd(const LinBwdArgs &a, int *grid_out, cudaStream_t s) {
     constexpr int cols = (nacc_d + TC_SPLIT_ACC) * 2 * KP;
     const int grid = tc_grid(a.N, smem, cols <= 128 ? 128 : (cols <= 256 ? 256 : 512), NT_BWD);
     DN_CUDA(cudaFuncSetAttribute(lin_bwd_kernel<KP, MP, RING, NT_BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    DN_LAUNCH((lin_bwd_kernel<KP, MP, RING, NT_BWD>), grid, NT_BWD, smem, s, a);
+    lin_bwd_kernel<KP, MP, RING, NT_BWD><<<grid, NT_BWD, smem, s>>>(a);
     *grid_out = grid;
     return 0;
 }
@@ -1100,9 +1088,8 @@ int dn4gl_lin_fwd_f32(const float *X, int64_t N, int32_t K, const float *in_bn, 
     const bool ring_ok = (K % 4 == 0) && aligned16(X);
     int rc = 0, grid = 0;
     // warp-specialised pipeline (mlp_pipe.cu) whenever the slabs are 16-byte granular; it also merges the batch statistics
-    // after a grid rendezvous (no bn_finalize launch).  DN4GL_LIN_SERIAL=1 keeps the phase-serial kernels (A/B, debugging).
-    static const bool serial_only = getenv("DN4GL_LIN_SERIAL") != nullptr;
-    if (!serial_only && (M % 4 == 0) && aligned16(Y) && (bn_out == nullptr || counters != nullptr)) {
+    // after a grid rendezvous (no bn_finalize launch)
+    if ((M % 4 == 0) && aligned16(Y) && (bn_out == nullptr || counters != nullptr)) {
         a.x_direct = (ring_ok && aligned16(W)) ? 0 : 1;     // e.g. the 2-feature first layer: X / W through bounds-checked loads
         BnFinalArgs f;
         f.gamma = gamma; f.beta = beta; f.eps = eps; f.momentum = momentum; f.bn_out = bn_out;
@@ -1117,7 +1104,7 @@ int dn4gl_lin_fwd_f32(const float *X, int64_t N, int32_t K, const float *in_bn, 
 #undef DN_FWD_CASE
     if (rc) return rc;
     if (bn_out != nullptr) {
-        DN_LAUNCH(bn_finalize_kernel, MP / 32, 1024, 0, s, reinterpret_cast<const float4 *>(a.part), grid, MP, M, N, gamma, beta, eps,
+        bn_finalize_kernel<<<MP / 32, 1024, 0, s>>>(reinterpret_cast<const float4 *>(a.part), grid, MP, M, N, gamma, beta, eps,
                                                     momentum, bn_out, running_mean, running_var,
                                                     reinterpret_cast<long long *>(num_batches_tracked));
         DN_LAUNCHED_N(2);
@@ -1157,10 +1144,9 @@ int dn4gl_lin_bwd_f32(const float *G, const float *Gseg, const int32_t *row2seg,
     const bool ring_ok = (K % 4 == 0) && (M % 4 == 0) && aligned16(X) && (G == nullptr || aligned16(G)) && (Yout == nullptr || aligned16(Yout));
     int rc = 0, grid = 0;
     // warp-specialised pipeline, partials merged after a grid rendezvous (mlp_pipe.cu): no lin_bwd_reduce launch
-    static const bool serial_only = getenv("DN4GL_LIN_SERIAL") != nullptr;
     const bool gy_ok = (M % 4 == 0) && (G == nullptr || aligned16(G)) && (Yout == nullptr || aligned16(Yout));
     const bool x_ok = (K % 4 == 0) && aligned16(X) && aligned16(W);
-    if (!serial_only && gy_ok && counters != nullptr && (x_ok || GX == nullptr) && (GX == nullptr || aligned16(GX)) &&
+    if (gy_ok && counters != nullptr && (x_ok || GX == nullptr) && (GX == nullptr || aligned16(GX)) &&
         (Gseg == nullptr || (aligned16(Gseg) && aligned16(row2seg)))) {
         a.x_direct = x_ok ? 0 : 1;
         const int g = dn4gl_pipe_lin_bwd(a, dW, db, sums_prev, ws, counters, s);
@@ -1173,7 +1159,7 @@ int dn4gl_lin_bwd_f32(const float *G, const float *Gseg, const int32_t *row2seg,
 #undef DN_BWD_CASE
     if (rc) return rc;
     const int elems = MP * KP + MP + 2 * KP;
-    DN_LAUNCH(lin_bwd_reduce_kernel, (elems + 31) / 32, 1024, 0, s, a.part, grid, MP, KP, M, K, dW, db, sums_prev);
+    lin_bwd_reduce_kernel<<<(elems + 31) / 32, 1024, 0, s>>>(a.part, grid, MP, KP, M, K, dW, db, sums_prev);
     DN_LAUNCHED_N(2);
     return DN4GL_OK;
 }
@@ -1186,7 +1172,7 @@ int dn4gl_bn_act_f32(const float *Y, int64_t N, int32_t M, const float *bn, int3
     const int64_t total = N * ((M + 3) / 4);
     const int64_t want = ceil_div64(total, 256 * 4);
     const int64_t cap = static_cast<int64_t>(dn4gl_num_sms()) * 8;
-    DN_LAUNCH(bn_act_kernel, static_cast<int>(want < cap ? want : cap), 256, 0, as_stream(stream), Y, N, M, bn, act, slope, out);
+    bn_act_kernel<<<static_cast<int>(want < cap ? want : cap), 256, 0, as_stream(stream)>>>(Y, N, M, bn, act, slope, out);
     DN_LAUNCHED();
     return DN4GL_OK;
 }
@@ -1204,12 +1190,12 @@ int dn4gl_bn_act_pool_f32(const float *Y, int64_t N, int32_t M, const float *bn,
     const int grid = B < cap ? B : cap;
     cudaStream_t s = as_stream(stream);
     switch (CHP) {
-    case 1: DN_LAUNCH(bn_act_pool_kernel<1>, grid, 256, 0, s, Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
-    case 2: DN_LAUNCH(bn_act_pool_kernel<2>, grid, 256, 0, s, Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
-    case 4: DN_LAUNCH(bn_act_pool_kernel<4>, grid, 256, 0, s, Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
-    case 8: DN_LAUNCH(bn_act_pool_kernel<8>, grid, 256, 0, s, Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
-    case 16: DN_LAUNCH(bn_act_pool_kernel<16>, grid, 256, 0, s, Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
-    default: DN_LAUNCH(bn_act_pool_kernel<32>, grid, 256, 0, s, Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
+    case 1: bn_act_pool_kernel<1><<<grid, 256, 0, s>>>(Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
+    case 2: bn_act_pool_kernel<2><<<grid, 256, 0, s>>>(Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
+    case 4: bn_act_pool_kernel<4><<<grid, 256, 0, s>>>(Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
+    case 8: bn_act_pool_kernel<8><<<grid, 256, 0, s>>>(Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
+    case 16: bn_act_pool_kernel<16><<<grid, 256, 0, s>>>(Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
+    default: bn_act_pool_kernel<32><<<grid, 256, 0, s>>>(Y, M, bn, act, slope, out, seg_ptr, B, mode, pooled); break;
     }
     DN_LAUNCHED();
     return DN4GL_OK;
@@ -1219,7 +1205,7 @@ int dn4gl_segment_ids_i32(const int32_t *seg_ptr, int32_t B, int64_t N, int32_t 
     DN_ARG(B >= 0 && N >= 0);
     if (N == 0) return DN4GL_OK;
     DN_ARG(seg_ptr != nullptr && out != nullptr && B >= 1);
-    DN_LAUNCH(segment_ids_kernel, static_cast<unsigned>(ceil_div64(N, 256)), 256, 0, as_stream(stream), seg_ptr, B, N, out);
+    segment_ids_kernel<<<static_cast<unsigned>(ceil_div64(N, 256)), 256, 0, as_stream(stream)>>>(seg_ptr, B, N, out);
     DN_LAUNCHED();
     return DN4GL_OK;
 }
@@ -1235,7 +1221,7 @@ int dn4gl_dot_f32(const float *a, const float *b, int64_t n, float *out, void *w
     DN_ARG(ws_bytes >= dn4gl_dot_workspace_bytes(n));
     const int64_t want = ceil_div64(n > 0 ? n : 1, 256 * 16);
     const int64_t cap = static_cast<int64_t>(dn4gl_num_sms()) * 4;
-    DN_LAUNCH(dot_kernel, static_cast<int>(want < cap ? want : cap), 256, 0, as_stream(stream), a, b, n, out, static_cast<float *>(ws), counter);
+    dot_kernel<<<static_cast<int>(want < cap ? want : cap), 256, 0, as_stream(stream)>>>(a, b, n, out, static_cast<float *>(ws), counter);
     DN_LAUNCHED();
     return DN4GL_OK;
 }
@@ -1310,15 +1296,15 @@ int dn4gl_bn_stats_f32(const float *Y, int64_t N, int32_t M, const float *gamma,
     const int grid = static_cast<int>(want < cap ? (want < 1 ? 1 : want) : cap);       // <= groups: every CTA has a first row
     float4 *part = static_cast<float4 *>(ws);
     switch (CHP) {
-    case 1: DN_LAUNCH(bn_stats_partial_kernel<1>, grid, 256, 0, s, Y, N, M, MP, part); break;
-    case 2: DN_LAUNCH(bn_stats_partial_kernel<2>, grid, 256, 0, s, Y, N, M, MP, part); break;
-    case 4: DN_LAUNCH(bn_stats_partial_kernel<4>, grid, 256, 0, s, Y, N, M, MP, part); break;
-    case 8: DN_LAUNCH(bn_stats_partial_kernel<8>, grid, 256, 0, s, Y, N, M, MP, part); break;
-    case 16: DN_LAUNCH(bn_stats_partial_kernel<16>, grid, 256, 0, s, Y, N, M, MP, part); break;
-    default: DN_LAUNCH(bn_stats_partial_kernel<32>, grid, 256, 0, s, Y, N, M, MP, part); break;
+    case 1: bn_stats_partial_kernel<1><<<grid, 256, 0, s>>>(Y, N, M, MP, part); break;
+    case 2: bn_stats_partial_kernel<2><<<grid, 256, 0, s>>>(Y, N, M, MP, part); break;
+    case 4: bn_stats_partial_kernel<4><<<grid, 256, 0, s>>>(Y, N, M, MP, part); break;
+    case 8: bn_stats_partial_kernel<8><<<grid, 256, 0, s>>>(Y, N, M, MP, part); break;
+    case 16: bn_stats_partial_kernel<16><<<grid, 256, 0, s>>>(Y, N, M, MP, part); break;
+    default: bn_stats_partial_kernel<32><<<grid, 256, 0, s>>>(Y, N, M, MP, part); break;
     }
-    DN_LAUNCH(bn_finalize_kernel, MP / 32, 1024, 0, s, reinterpret_cast<const float4 *>(part), grid, MP, M, N, gamma, beta, eps, momentum,
-              bn_out, running_mean, running_var, reinterpret_cast<long long *>(num_batches_tracked));
+    bn_finalize_kernel<<<MP / 32, 1024, 0, s>>>(reinterpret_cast<const float4 *>(part), grid, MP, M, N, gamma, beta, eps, momentum,
+                                                bn_out, running_mean, running_var, reinterpret_cast<long long *>(num_batches_tracked));
     DN_LAUNCHED_N(2);
     return DN4GL_OK;
 }
@@ -1333,12 +1319,12 @@ int dn4gl_bn_bwd_apply_f32(const float *G, const float *Y, int64_t N, int32_t M,
     const int64_t want = ceil_div64(N, static_cast<int64_t>(RP) * 4), cap = static_cast<int64_t>(dn4gl_num_sms()) * 8;
     const int grid = static_cast<int>(want < cap ? (want < 1 ? 1 : want) : cap);
     switch (CHP) {
-    case 1: DN_LAUNCH(bn_bwd_apply_kernel<1>, grid, 256, 0, s, G, Y, N, M, bn, sums, act, slope, GX); break;
-    case 2: DN_LAUNCH(bn_bwd_apply_kernel<2>, grid, 256, 0, s, G, Y, N, M, bn, sums, act, slope, GX); break;
-    case 4: DN_LAUNCH(bn_bwd_apply_kernel<4>, grid, 256, 0, s, G, Y, N, M, bn, sums, act, slope, GX); break;
-    case 8: DN_LAUNCH(bn_bwd_apply_kernel<8>, grid, 256, 0, s, G, Y, N, M, bn, sums, act, slope, GX); break;
-    case 16: DN_LAUNCH(bn_bwd_apply_kernel<16>, grid, 256, 0, s, G, Y, N, M, bn, sums, act, slope, GX); break;
-    default: DN_LAUNCH(bn_bwd_apply_kernel<32>, grid, 256, 0, s, G, Y, N, M, bn, sums, act, slope, GX); break;
+    case 1: bn_bwd_apply_kernel<1><<<grid, 256, 0, s>>>(G, Y, N, M, bn, sums, act, slope, GX); break;
+    case 2: bn_bwd_apply_kernel<2><<<grid, 256, 0, s>>>(G, Y, N, M, bn, sums, act, slope, GX); break;
+    case 4: bn_bwd_apply_kernel<4><<<grid, 256, 0, s>>>(G, Y, N, M, bn, sums, act, slope, GX); break;
+    case 8: bn_bwd_apply_kernel<8><<<grid, 256, 0, s>>>(G, Y, N, M, bn, sums, act, slope, GX); break;
+    case 16: bn_bwd_apply_kernel<16><<<grid, 256, 0, s>>>(G, Y, N, M, bn, sums, act, slope, GX); break;
+    default: bn_bwd_apply_kernel<32><<<grid, 256, 0, s>>>(G, Y, N, M, bn, sums, act, slope, GX); break;
     }
     DN_LAUNCHED();
     return DN4GL_OK;

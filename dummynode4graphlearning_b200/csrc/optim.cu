@@ -29,7 +29,6 @@ __global__ void __launch_bounds__(256) adam_kernel(float *__restrict__ p, const 
                                                    float *__restrict__ v, float *__restrict__ vmax, int64_t n,
                                                    const float *__restrict__ hyper, float *step, int decoupled,
                                                    int32_t *counter) {
-    DN_PDL_WAIT();
     const AdamHyper h = {hyper[0], hyper[1], hyper[2], hyper[3], hyper[4]};
     // bias corrections in double, once per CTA (pow is ~200 FP64 instructions)
     __shared__ float sh_step_size, sh_inv_bc2_sqrt, sh_t;
@@ -85,7 +84,7 @@ extern "C" int dn4gl_adam_f32(float *param, const float *grad, float *exp_avg, f
     const int64_t cap = static_cast<int64_t>(dn4gl_num_sms()) * 8;
     if (want > cap) want = cap;
     if (want < 1) want = 1;
-    DN_LAUNCH(adam_kernel, static_cast<unsigned>(want), 256, 0, as_stream(stream), param, grad, exp_avg, exp_avg_sq, max_exp_avg_sq, n,
+    adam_kernel<<<static_cast<unsigned>(want), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, max_exp_avg_sq, n,
                                                                             hyper, step, decoupled, counter);
     DN_LAUNCHED();
     return DN4GL_OK;

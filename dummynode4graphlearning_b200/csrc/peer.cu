@@ -49,7 +49,6 @@ __device__ __forceinline__ float4 ld_sys_v4(const float *p) {      // coherent a
 template <int W>
 __global__ void __launch_bounds__(256) peer_allreduce_kernel(PeerPtrs pp, int rank, int64_t n4, float weight,
                                                              float4 *__restrict__ bucket) {
-    DN_PDL_WAIT();
     constexpr int world = W;
     int32_t *mine = pp.sig[rank];
     const int b = static_cast<int>(blockIdx.x), t = static_cast<int>(threadIdx.x);
@@ -127,14 +126,14 @@ extern "C" int dn4gl_peer_allreduce_f32(float *bucket, int64_t n, float weight, 
     float4 *b4 = reinterpret_cast<float4 *>(bucket);
     const int rk = static_cast<int>(rank);
     switch (world) {
-    case 1: DN_LAUNCH(peer_allreduce_kernel<1>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    case 2: DN_LAUNCH(peer_allreduce_kernel<2>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    case 3: DN_LAUNCH(peer_allreduce_kernel<3>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    case 4: DN_LAUNCH(peer_allreduce_kernel<4>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    case 5: DN_LAUNCH(peer_allreduce_kernel<5>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    case 6: DN_LAUNCH(peer_allreduce_kernel<6>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    case 7: DN_LAUNCH(peer_allreduce_kernel<7>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
-    default: DN_LAUNCH(peer_allreduce_kernel<8>, grid, 256, 0, st, pp, rk, n / 4, weight, b4); break;
+    case 1: peer_allreduce_kernel<1><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    case 2: peer_allreduce_kernel<2><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    case 3: peer_allreduce_kernel<3><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    case 4: peer_allreduce_kernel<4><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    case 5: peer_allreduce_kernel<5><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    case 6: peer_allreduce_kernel<6><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    case 7: peer_allreduce_kernel<7><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
+    default: peer_allreduce_kernel<8><<<grid, 256, 0, st>>>(pp, rk, n / 4, weight, b4); break;
     }
     DN_LAUNCHED();
     return DN4GL_OK;

@@ -27,11 +27,6 @@
 // bit-identical to the per-row kernel and to the sequential oracle.
 #include "common.cuh"
 
-// Tiling refinements measured in round 2 (profiles/r2a_k1_c2_*.jsonl, r2l_bench.json; C2 structure): whole-graph tiles
-// (-DDN4GL_TILE_WHOLE_GRAPHS) change nothing by themselves (24.5 vs 24.6 us cold); the cost-balanced deal
-// (-DDN4GL_TILE_BALANCE) brings the kernel from 21.5 to 18.8 us back to back, but its one-CTA sort + greedy assignment
-// costs ~300 us per tiling -- per mini-batch, twice -- so it only pays for a structure that is reused for many launches.
-// Both stay compiled out of the product build.
 constexpr int TP_NCW_MAX = 31;                // consumer warps: 15 (512 threads, <=128 registers) or 31 (1024 threads, 64)
 constexpr int TP_SPLIT = 64;                  // rows above this many neighbours are split (== graph.py HEAVY_THRESHOLD)
 constexpr int TP_MAX_STAGES = 4;
@@ -282,35 +277,12 @@ __device__ __forceinline__ void process_tile_fast(const TileAddr<LANES, VEC> &ta
                     add4(acc[k], v0); add4(acc[k], v1); add4(acc[k], v2); add4(acc[k], v3);
                 }
             }
-#ifdef DN4GL_K1_TAIL_ILP
-            // EXPERIMENT (off in the product build, `make libdn4gl_exp.so`): the 1..3 neighbours left after the
-            // four-wide batches are fetched together -- all index loads, then all row loads, then the adds in CSR
-            // order (bit-identical result) -- instead of one dependent col -> x -> add chain per neighbour.  Absent
-            // neighbours re-read the first one (a valid address) and are not added.
-            {
-                const int rem = static_cast<int>(ce - ca) >> 2;   // 0..3
-                if (rem > 0) {
-                    const uint32_t c0 = static_cast<uint32_t>(lds32(ca));
-                    const uint32_t c1 = rem > 1 ? static_cast<uint32_t>(lds32(ca + 4u)) : c0;
-                    const uint32_t c2 = rem > 2 ? static_cast<uint32_t>(lds32(ca + 8u)) : c0;
-                    const uint32_t a0 = xa + c0 * ROWB, a1 = xa + c1 * ROWB, a2 = xa + c2 * ROWB;
-#pragma unroll
-                    for (int k = 0; k < VEC; ++k) {
-                        const float4 v0 = lds128(a0 + k * KB), v1 = lds128(a1 + k * KB), v2 = lds128(a2 + k * KB);
-                        add4(acc[k], v0);
-                        if (rem > 1) add4(acc[k], v1);
-                        if (rem > 2) add4(acc[k], v2);
-                    }
-                }
-            }
-#else
 #pragma unroll 1
             for (; ca < ce; ca += 4u) {
                 const uint32_t a0 = xa + static_cast<uint32_t>(lds32(ca)) * ROWB;
 #pragma unroll
                 for (int k = 0; k < VEC; ++k) add4(acc[k], lds128(a0 + k * KB));
             }
-#endif
             if (self_scale != 0.f) {
                 const uint32_t a0 = xa + static_cast<uint32_t>(row) * ROWB;
 #pragma unroll
@@ -350,145 +322,6 @@ __device__ __forceinline__ void process_tile_fast(const TileAddr<LANES, VEC> &ta
         }
     }
 }
-
-#ifdef DN4GL_K1_TWO_ROWS
-// EXPERIMENT (off in the product build; `make libdn4gl_exp.so EXP_FLAGS=-DDN4GL_K1_TWO_ROWS`): process_tile_fast with
-// TWO rows per sub-group in flight -- the row_ptr pairs of both rows are fetched together and the four-wide batches of
-// both rows are issued together (8 index loads, 8 row loads before the first add), so that the dependent
-// row_ptr -> col -> x chain at the start of a row overlaps with the other row's.  Per-row accumulation order is
-// unchanged (CSR order), i.e. the result is bit-identical; what is left of the longer row runs through the single-row
-// loops.  Long rows (> TP_SPLIT) are split over the warp's sub-groups exactly as in process_tile_fast.
-template <int LANES, int VEC, int NCW>
-__device__ __forceinline__ void process_tile_fast2(const TileAddr<LANES, VEC> &ta, float4 *__restrict__ out,
-                                                   float self_scale, int cw, int lane) {
-    constexpr int RPW = 32 / LANES;
-    constexpr int DV = LANES * VEC;
-    constexpr uint32_t ROWB = DV * 16u;
-    constexpr uint32_t KB = LANES * 16u;
-    constexpr int STEP = NCW * RPW;
-    const int sub = lane / LANES, sl = lane % LANES;
-    const uint32_t xa = ta.x_a, ca_base = ta.col_a;
-    float4 *outl = out + sl;
-#pragma unroll 1
-    for (int rb = ta.r0 + cw * RPW; rb < ta.r1; rb += 2 * STEP) {
-        int row[2], beg[2], end[2];
-        bool valid[2], big[2], run[2];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            row[h] = rb + h * STEP + sub;
-            valid[h] = row[h] < ta.r1;
-            beg[h] = 0;
-            end[h] = 0;
-        }
-#pragma unroll
-        for (int h = 0; h < 2; ++h)
-            if (valid[h]) {
-                const uint32_t ra = ta.rp_a + 4u * static_cast<uint32_t>(row[h]);
-                beg[h] = lds32(ra);
-                end[h] = lds32(ra + 4u);
-            }
-        float4 acc[2][VEC];
-        uint32_t ca[2], ce[2];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            big[h] = (LANES < 32) && (end[h] - beg[h] > TP_SPLIT);
-            run[h] = valid[h] && !big[h];
-            ca[h] = ca_base + 4u * static_cast<uint32_t>(beg[h]);
-            ce[h] = run[h] ? ca_base + 4u * static_cast<uint32_t>(end[h]) : ca[h];   // empty range when not run here
-#pragma unroll
-            for (int k = 0; k < VEC; ++k) acc[h][k] = zero4();
-        }
-#pragma unroll 1
-        while (ca[0] + 16u <= ce[0] && ca[1] + 16u <= ce[1]) {   // both rows: 4 + 4 neighbours in flight
-            uint32_t a[2][4];
-#pragma unroll
-            for (int h = 0; h < 2; ++h)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) a[h][j] = xa + static_cast<uint32_t>(lds32(ca[h] + 4u * j)) * ROWB;
-#pragma unroll
-            for (int k = 0; k < VEC; ++k) {
-                float4 v[2][4];
-#pragma unroll
-                for (int h = 0; h < 2; ++h)
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) v[h][j] = lds128(a[h][j] + k * KB);
-#pragma unroll
-                for (int h = 0; h < 2; ++h)
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) add4(acc[h][k], v[h][j]);
-            }
-            ca[0] += 16u;
-            ca[1] += 16u;
-        }
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {   // what is left of either row
-#pragma unroll 1
-            for (; ca[h] + 16u <= ce[h]; ca[h] += 16u) {
-                const uint32_t a0 = xa + static_cast<uint32_t>(lds32(ca[h])) * ROWB;
-                const uint32_t a1 = xa + static_cast<uint32_t>(lds32(ca[h] + 4u)) * ROWB;
-                const uint32_t a2 = xa + static_cast<uint32_t>(lds32(ca[h] + 8u)) * ROWB;
-                const uint32_t a3 = xa + static_cast<uint32_t>(lds32(ca[h] + 12u)) * ROWB;
-#pragma unroll
-                for (int k = 0; k < VEC; ++k) {
-                    const float4 v0 = lds128(a0 + k * KB), v1 = lds128(a1 + k * KB);
-                    const float4 v2 = lds128(a2 + k * KB), v3 = lds128(a3 + k * KB);
-                    add4(acc[h][k], v0); add4(acc[h][k], v1); add4(acc[h][k], v2); add4(acc[h][k], v3);
-                }
-            }
-#pragma unroll 1
-            for (; ca[h] < ce[h]; ca[h] += 4u) {
-                const uint32_t a0 = xa + static_cast<uint32_t>(lds32(ca[h])) * ROWB;
-#pragma unroll
-                for (int k = 0; k < VEC; ++k) add4(acc[h][k], lds128(a0 + k * KB));
-            }
-        }
-#pragma unroll
-        for (int h = 0; h < 2; ++h)
-            if (run[h]) {
-                if (self_scale != 0.f) {
-                    const uint32_t a0 = xa + static_cast<uint32_t>(row[h]) * ROWB;
-#pragma unroll
-                    for (int k = 0; k < VEC; ++k) axpy4_rn(acc[h][k], self_scale, lds128(a0 + k * KB));
-                }
-                float4 *o = outl + static_cast<int64_t>(row[h]) * DV;
-#pragma unroll
-                for (int k = 0; k < VEC; ++k) o[k * LANES] = acc[h][k];
-            }
-        if constexpr (LANES < 32) {
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                unsigned m = __ballot_sync(0xffffffffu, valid[h] && big[h]);
-                while (m) {   // long rows of this half-iteration, split over the RPW sub-groups of the warp
-                    const int src_lane = __ffs(m) - 1;
-                    m &= ~(((1u << LANES) - 1u) << src_lane);
-                    const int brow = rb + h * STEP + src_lane / LANES;
-                    const int bbeg = __shfl_sync(0xffffffffu, beg[h], src_lane);
-                    const int bend = __shfl_sync(0xffffffffu, end[h], src_lane);
-                    float4 bacc = zero4();
-                    uint32_t cb = ca_base + 4u * static_cast<uint32_t>(bbeg + sub);
-                    const uint32_t cbe = ca_base + 4u * static_cast<uint32_t>(bend);
-#pragma unroll 1
-                    for (; cb + 12u * RPW < cbe; cb += 16u * RPW) {
-                        const uint32_t a0 = xa + static_cast<uint32_t>(lds32(cb)) * ROWB;
-                        const uint32_t a1 = xa + static_cast<uint32_t>(lds32(cb + 4u * RPW)) * ROWB;
-                        const uint32_t a2 = xa + static_cast<uint32_t>(lds32(cb + 8u * RPW)) * ROWB;
-                        const uint32_t a3 = xa + static_cast<uint32_t>(lds32(cb + 12u * RPW)) * ROWB;
-                        const float4 v0 = lds128(a0), v1 = lds128(a1), v2 = lds128(a2), v3 = lds128(a3);
-                        add4(bacc, v0); add4(bacc, v1); add4(bacc, v2); add4(bacc, v3);
-                    }
-#pragma unroll 1
-                    for (; cb < cbe; cb += 4u * RPW) add4(bacc, lds128(xa + static_cast<uint32_t>(lds32(cb)) * ROWB));
-                    subgroup_allreduce<LANES>(bacc);
-                    if (sub == 0) {
-                        if (self_scale != 0.f) axpy4_rn(bacc, self_scale, lds128(xa + static_cast<uint32_t>(brow) * ROWB));
-                        outl[static_cast<int64_t>(brow) * DV] = bacc;
-                    }
-                }
-            }
-        }
-    }
-}
-#endif
 
 // one listed long row of a cut tile, reduced by all consumer warps of the CTA through `scratch` (an idle stage)
 template <int LANES, int VEC, int NCW>
@@ -563,9 +396,7 @@ spmm_pipe_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict_
                  const int32_t *__restrict__ heavy_list, const int32_t *__restrict__ heavy_count, float self_scale,
                  const float *__restrict__ eps_dev, int smem_bytes, int stages, int nnz_per_row) {
     constexpr int DV = LANES * VEC;
-#ifndef DN4GL_PDL
     if (eps_dev != nullptr) self_scale = 1.f + __ldg(eps_dev);   // trainable GIN eps lives on the device
-#endif
     if (threadIdx.x == 32) TL_STAMP(0);
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ uint64_t full_bar[TP_MAX_STAGES], empty_bar[TP_MAX_STAGES];
@@ -579,10 +410,6 @@ spmm_pipe_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict_
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
-#ifdef DN4GL_PDL
-    DN_PDL_WAIT();   // (experiment) barrier set-up above overlaps the previous kernel's tail; global memory from here on
-    if (eps_dev != nullptr) self_scale = 1.f + __ldg(eps_dev);
-#endif
     const int H = (heavy_list != nullptr && heavy_count != nullptr) ? __ldg(heavy_count) : 0;
     const int total = H + num_tiles;
     if (threadIdx.x == 32) TL_STAMP(1);
@@ -658,11 +485,7 @@ spmm_pipe_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restrict_
                     ta.r0 = td.x; ta.r1 = td.y; ta.e0 = td.z; ta.nst = min(nnz, L.cap_nnz);
                 }
                 if (rows <= L.cap_rows && !open && nnz <= L.cap_nnz)
-#ifdef DN4GL_K1_TWO_ROWS
-                    process_tile_fast2<LANES, VEC, NCW>(ta, out, self_scale, cw, lane);
-#else
                     process_tile_fast<LANES, VEC, NCW>(ta, out, self_scale, cw, lane);
-#endif
                 else if (rows <= L.cap_rows)
                     process_tile<LANES, VEC, NCW, true>(ta, row_ptr, col, x, out, self_scale, cut, cw, lane);
                 else
@@ -691,18 +514,6 @@ __device__ __forceinline__ int tile_boundary(const int32_t *__restrict__ seg_ptr
     }
     const int gs = seg_ptr[lo];
     if (gs < target + C) { *aligned = true; return gs; }
-#ifdef DN4GL_TILE_WHOLE_GRAPHS
-    // EXPERIMENT (off in the product build; `make libdn4gl_exp.so EXP_FLAGS=-DDN4GL_TILE_WHOLE_GRAPHS`, host model and
-    // invariants: tools/k1_tiles_model.py).  Window k lies inside graph lo - 1 = [s, e).  If that graph fits one stage
-    // (rows <= 2 C <= cap_rows) it is not cut: the spanned window's slot -- otherwise an arbitrary cut -- starts at the
-    // graph's first row, so tile k - 1 ends there and tile k = [s, e) is the whole graph (closed, unchecked fast path).
-    // C2: rows in cut tiles 15.2 % -> 5.8 %.  Boundaries stay non-decreasing and every tile still lies within one
-    // window of its slot; anything this gets wrong is caught as before (verify_tiles_kernel, capacity checks).
-    if (lo >= 1) {
-        const int s = seg_ptr[lo - 1];
-        if (gs - s <= 2 * C) { *aligned = true; return (k == s / C + 1) ? s : gs; }
-    }
-#endif
     *aligned = false;
     return static_cast<int>(target);
 }
@@ -743,106 +554,11 @@ __global__ void collect_cut_heavy_kernel(const int32_t *__restrict__ row_ptr, in
     int k = r / C;
     if (k >= T) k = T - 1;
     if (r < tiles[k].x) --k;
-#ifdef DN4GL_TILE_WHOLE_GRAPHS
-    else if (r >= tiles[k].y && k + 1 < T) ++k;   // the next slot's tile may start inside this window
-#endif
     if (tiles[k].w < 0) {
         const int i = atomicAdd(heavy_count, 1);
         if (i < cap) heavy_list[i] = r;
     }
 }
-
-#ifdef DN4GL_TILE_BALANCE
-// EXPERIMENT (off in the product build; `make libdn4gl_exp_balance.so`, host model: tools/k1_tiles_model.py).  The pipe
-// kernel deals its work items round-robin: CTA b takes the items t with t % G == b, the H listed long rows first, then the
-// tiles in row order -- at C2 the estimated spread of the CTA loads is 1.7-2.2x the mean and the slowest CTA is the
-// kernel's duration.  This kernel PERMUTES the tile descriptors in place (the pipe kernel does not care about their
-// order) so that the same deal hands every CTA about the same work: tiles sorted by estimated cost, longest first, each
-// given to the least-loaded CTA that still has a free slot (CTA b owns the slots i with (H + i) % G == b); model:
-// 1.12-1.25x.  One CTA, T <= TB_MAX descriptors held in shared memory; runs once per tiling, after the long-row list has
-// been collected (that step looks tiles up by window).
-constexpr int TB_MAX = 1024;
-__device__ __forceinline__ int tb_tile_cost(const int4 td) {
-    const int rows = td.y - td.x, nnz = (td.w & 0x7fffffff) - td.z;
-    const int c = (nnz >> 2) + rows;                 // four-neighbour batches + per-row overhead
-    return td.w < 0 ? 2 * c : c;                     // rows of cut tiles take the checked path
-}
-__global__ void __launch_bounds__(1024)
-balance_tiles_kernel(int4 *__restrict__ tiles, int T, const int32_t *__restrict__ row_ptr,
-                     const int32_t *__restrict__ heavy_list, const int32_t *__restrict__ heavy_count, int G) {
-    __shared__ int4 desc[TB_MAX];
-    __shared__ unsigned long long key[TB_MAX];       // (cost << 32) | (0xffffffff - index): descending sort, stable
-    __shared__ int dest[TB_MAX];
-    __shared__ int load[256], freec[256], used[256];
-    const int tid = threadIdx.x;
-    int P = 1;
-    while (P < T) P <<= 1;
-    for (int i = tid; i < P; i += blockDim.x) {
-        unsigned long long k = 0ull;
-        if (i < T) {
-            const int4 td = tiles[i];
-            desc[i] = td;
-            k = (static_cast<unsigned long long>(static_cast<unsigned>(tb_tile_cost(td))) << 32) |
-                static_cast<unsigned long long>(0xffffffffu - static_cast<unsigned>(i));
-        }
-        key[i] = k;
-    }
-    const int H = (heavy_list != nullptr && heavy_count != nullptr) ? *heavy_count : 0;
-    for (int b = tid; b < G; b += blockDim.x) {
-        const int first = ((b - H % G) % G + G) % G;          // first tile slot i with (H + i) % G == b
-        load[b] = 0;
-        used[b] = 0;
-        freec[b] = first < T ? (T - 1 - first) / G + 1 : 0;
-    }
-    __syncthreads();
-    for (int i = tid; i < H; i += blockDim.x) {                // the listed long rows keep their places
-        const int r = heavy_list[i];
-        atomicAdd(&load[i % G], ((row_ptr[r + 1] - row_ptr[r]) >> 2) + 256);
-    }
-    for (int k2 = 2; k2 <= P; k2 <<= 1) {                      // bitonic sort, descending
-        for (int j = k2 >> 1; j > 0; j >>= 1) {
-            __syncthreads();
-            for (int i = tid; i < P; i += blockDim.x) {
-                const int l = i ^ j;
-                if (l > i) {
-                    const unsigned long long a = key[i], c = key[l];
-                    const bool desc_run = (i & k2) == 0;
-                    if (desc_run ? (a < c) : (a > c)) { key[i] = c; key[l] = a; }
-                }
-            }
-        }
-    }
-    __syncthreads();
-    if (tid < 32) {                                            // greedy longest-first, one warp, items in sorted order
-        for (int k = 0; k < T; ++k) {
-            unsigned long long best = ~0ull;                   // (load << 32) | b of the least-loaded CTA with a free slot
-            for (int b = tid; b < G; b += 32)
-                if (freec[b] > 0) {
-                    const unsigned long long v = (static_cast<unsigned long long>(static_cast<unsigned>(load[b])) << 32) |
-                                                 static_cast<unsigned>(b);
-                    best = v < best ? v : best;
-                }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                const unsigned long long v = __shfl_xor_sync(0xffffffffu, best, o);
-                best = v < best ? v : best;
-            }
-            if (tid == 0) {
-                const int b = static_cast<int>(best & 0xffffffffu);
-                const int first = ((b - H % G) % G + G) % G;
-                dest[k] = first + used[b] * G;
-                used[b] += 1;
-                freec[b] -= 1;
-                load[b] += static_cast<int>(key[k] >> 32);
-            }
-            __syncwarp();
-        }
-    }
-    __syncthreads();
-    for (int k = tid; k < T; k += blockDim.x)
-        tiles[dest[k]] = desc[0xffffffffu - static_cast<unsigned>(key[k] & 0xffffffffu)];
-}
-#endif
 
 extern "C" int dn4gl_make_row_tiles(const int32_t *seg_ptr, int32_t B, int32_t window_rows, const int32_t *row_ptr,
                                     const int32_t *col, int64_t N, int32_t *tile_desc, int32_t num_tiles,
@@ -866,16 +582,6 @@ extern "C" int dn4gl_make_row_tiles(const int32_t *seg_ptr, int32_t B, int32_t w
                 heavy_cap, heavy_count);
             ++launched;
         }
-#ifdef DN4GL_TILE_BALANCE
-        {
-            const int G = dn4gl_num_sms();
-            if (num_tiles > G && num_tiles <= TB_MAX && G <= 256) {
-                balance_tiles_kernel<<<1, 1024, 0, st>>>(reinterpret_cast<int4 *>(tile_desc), num_tiles, row_ptr, heavy_list,
-                                                         heavy_count, G);
-                ++launched;
-            }
-        }
-#endif
     }
     if (launched) DN_LAUNCHED_N(launched);
     return DN4GL_OK;
@@ -902,7 +608,7 @@ static int launch_pipe(const int32_t *row_ptr, const int32_t *col, const float *
     int64_t want = static_cast<int64_t>(num_tiles) + (heavy_list ? heavy_cap : 0);
     int grid = static_cast<int>(want < dn4gl_num_sms() ? want : dn4gl_num_sms());
     if (grid < 1) grid = 1;
-    DN_LAUNCH((spmm_pipe_kernel<LANES, VEC, NCW>), grid, (NCW + 1) * 32, smem_bytes, st,
+    spmm_pipe_kernel<LANES, VEC, NCW><<<grid, (NCW + 1) * 32, smem_bytes, st>>>(
         row_ptr, col, reinterpret_cast<const float4 *>(x), reinterpret_cast<float4 *>(out),
         reinterpret_cast<const int4 *>(tile_desc), num_tiles, heavy_list, heavy_count, self_scale, eps_dev, smem_bytes, stages,
         nnz_per_row);

@@ -1,7 +1,6 @@
 // Shared device helpers of the tensor-core MLP stage kernels (mlp_tc.cu, mlp_pipe.cu): tcgen05 / TMEM / mbarrier /
 // bulk-copy PTX wrappers, the 128-byte-swizzled operand tile layouts, the 3xTF32 split and the BatchNorm record.
 #pragma once
-#include <cstdlib>
 #include "common.cuh"
 
 // ---- argument blocks of the stage kernels (shared by the phase-serial kernels in mlp_tc.cu and the warp-specialised
@@ -332,10 +331,7 @@ static inline cudaError_t launch_coop(void (*kernel)(P...), int grid, int block,
     attr[0].id = cudaLaunchAttributeCooperative;
     attr[0].val.cooperative = 1;
     cfg.attrs = attr;
-    // DN4GL_NO_COOP=1 (measurement only -- without the attribute nothing guarantees that the waiting CTAs' peers are ever
-    // scheduled): what the cooperative launch itself costs, see DESIGN.md
-    static const bool plain = getenv("DN4GL_NO_COOP") != nullptr;
-    cfg.numAttrs = plain ? 0 : 1;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<P>(args)...);
 }
 

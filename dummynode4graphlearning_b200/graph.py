@@ -20,7 +20,6 @@ from ._lib import lib, ptr
 
 HEAVY_THRESHOLD = 64  # rows with more in-edges than this are reduced by a whole CTA (dummy nodes)
 TILE_SMEM = int(os.environ.get("DN4GL_TILE_SMEM", str(200 * 1024)))   # shared-memory ring of the pipelined aggregation kernel
-TILE_STAGES = os.environ.get("DN4GL_TILE_STAGES", "")                   # "" = chosen per batch (4, 3 or 2); "3" forces three stages
 TILE_WARPS = int(os.environ.get("DN4GL_TILE_WARPS", "32"))             # warps per CTA for D <= 128 (16 | 32)
 
 _dev_bound = {}
@@ -81,8 +80,7 @@ class CSR:
         L = lib()
         npr = min(max(-(-self.nnz // max(self.n_rows, 1)) + 1, 2), 32)
         stages = cap = None
-        forced = int(TILE_STAGES) if TILE_STAGES else None      # experiments only (tools/bench_k1_c2.py); default: automatic
-        for s in ((forced,) if forced else (4, 3, 2)):
+        for s in (4, 3, 2):
             c = L.size("dn4gl_spmm_tiled_cap_rows", D, smem_bytes, s, npr)
             if self.max_seg is None:
                 if s == 3:
@@ -92,7 +90,7 @@ class CSR:
                 stages, cap = s, c
                 break
         if stages is None:
-            stages = forced or 2
+            stages = 2
             cap = L.size("dn4gl_spmm_tiled_cap_rows", D, smem_bytes, stages, npr)
         aligned = self.max_seg is not None and 2 * self.max_seg <= cap
         window = max(cap - self.max_seg if aligned else cap // 2, 1)

@@ -42,9 +42,6 @@ int dn4gl_version(void);
 const char *dn4gl_last_error(void);
 /* binds the calling thread to `device` (cudaSetDevice); one process per GPU is the intended use */
 int dn4gl_set_device(int device);
-/* caps the SM count the library sizes its (persistent) grids with; 0 = all SMs.  Process-wide; set it before the first
- * workspace query / launch and leave it (workspace sizes depend on it).  Used to leave SMs to a concurrent stream.     */
-int dn4gl_set_sm_limit(int n);
 /* number of CUDA kernels this library has launched in this process so far (monotonic counter) */
 int64_t dn4gl_launch_count(void);
 

@@ -1,8 +1,7 @@
 """CPU: invariants of the aggregation kernel's tile construction on the host model (tools/k1_tiles_model.py restates
-csrc/spmm_tiled.cu tile_boundary / make_row_tiles_kernel / collect_cut_heavy_kernel): for the shipped rule and for the
-prepared whole-graph rule (-DDN4GL_TILE_WHOLE_GRAPHS) the tiles partition [0, N), closed tiles hold whole graphs and fit
-one stage, and the +-1 window search finds every row's tile.  The device code itself is covered by the GPU aggregation
-tests (tests/test_agg_gpu.py, every ring size)."""
+csrc/spmm_tiled.cu tile_boundary / make_row_tiles_kernel / collect_cut_heavy_kernel): the tiles partition [0, N), closed
+tiles hold whole graphs and fit one stage, and the window search finds every row's tile.  The device code itself is
+covered by the GPU aggregation tests (tests/test_agg_gpu.py, every ring size)."""
 import importlib.util
 import os
 
@@ -16,57 +15,18 @@ spec.loader.exec_module(model)
 
 
 @pytest.mark.parametrize("C", [1, 2, 7, 64, 311])
-def test_tiles_partition_rows_under_both_rules(C):
+def test_tiles_partition_rows(C):
     rng = np.random.default_rng(C)
     for trial in range(120):
         n = rng.integers(1, 4 * C + 2, int(rng.integers(1, 40)))
         if trial % 3 == 0:
             n = np.minimum(n, int(rng.integers(1, 2 * C + 2)))
         seg = np.concatenate([[0], np.cumsum(n)])
-        cut_old, _ = model.check(seg, C, whole=False)
-        cut_new, biggest = model.check(seg, C, whole=True)
-        assert cut_new <= cut_old + 1e-12        # the whole-graph rule never cuts more rows than the shipped one
+        _, biggest = model.check(seg, C)
         assert biggest <= 2 * C
 
 
-def test_whole_graph_rule_keeps_a_spanning_graph_in_one_tile():
-    # window 10; graphs of 8, 19 (spans window 1 = rows [10, 20)) and 3 rows: the shipped rule cuts the 19-row graph at 10
+def test_a_graph_longer_than_the_window_is_cut():
+    # window 10; graphs of 8, 19 (spans window 1 = rows [10, 20)) and 3 rows: the 19-row graph is cut at 10
     seg = np.array([0, 8, 27, 30])
-    assert model.make_tiles(seg, 10, whole=False) == [(0, 10, True), (10, 27, True), (27, 30, False)]
-    assert model.make_tiles(seg, 10, whole=True) == [(0, 8, False), (8, 27, False), (27, 30, False)]
-    # a graph longer than two windows is still cut
-    seg = np.array([0, 4, 29, 33])
-    assert any(cut for _, _, cut in model.make_tiles(seg, 10, whole=True))
-
-
-@pytest.mark.parametrize("seed", range(8))
-def test_balanced_deal_is_a_permutation_and_flattens_the_loads(seed):
-    """the greedy longest-first slot assignment of the prepared -DDN4GL_TILE_BALANCE experiment (restated in
-    tools/k1_tiles_model.py::device_balance): every tile lands in exactly one slot, every CTA keeps its slot count, and
-    the estimated load spread of the round-robin deal shrinks on heavy-tailed tile costs."""
-    rng = np.random.default_rng(seed)
-    G, T, H = 16, int(rng.integers(40, 200)), int(rng.integers(0, 10))
-    desc, e = [], 0
-    for k in range(T):
-        rows = int(rng.integers(0, 600))
-        nnz = int(rows * rng.integers(2, 9) + (rng.integers(0, 5) == 0) * rng.integers(0, 20000))
-        desc.append((1000 * k, 1000 * k + rows, e, e + nnz, bool(rng.integers(0, 6) == 0)))
-        e += nnz
-    heavy = [int(rng.integers(256, 600)) for _ in range(H)]
-    order, dest, load = model.device_balance(desc, H, heavy, G)
-    assert sorted(order) == list(range(T)) and sorted(dest) == list(range(T))
-    cost = {i: (((d[3] - d[2]) >> 2) + (d[1] - d[0])) * (2 if d[4] else 1) for i, d in enumerate(desc)}
-    # loads recomputed from the final layout under the kernel's deal: item t -> CTA t % G, long rows first
-    after = [0] * G
-    for i in range(H):
-        after[i % G] += heavy[i]
-    for k, slot in zip(order, dest):
-        after[(H + slot) % G] += cost[k]
-    assert after == load
-    before = [0] * G
-    for i in range(H):
-        before[i % G] += heavy[i]
-    for i in range(T):
-        before[(H + i) % G] += cost[i]
-    assert max(after) <= max(before)
-    assert max(after) <= 1.35 * (sum(after) / G) or max(after) == max(cost.values())
+    assert model.make_tiles(seg, 10) == [(0, 10, True), (10, 27, True), (27, 30, False)]

@@ -1,9 +1,7 @@
 """CPU model of the aggregation kernel's tile construction (csrc/spmm_tiled.cu: tile_boundary / make_row_tiles_kernel /
-collect_cut_heavy_kernel), no GPU: the shipped rule (graphs longer than the window are cut -> checked slow path) against
-the experiment -DDN4GL_TILE_WHOLE_GRAPHS (a graph that spans a window but fits one stage, rows <= 2 * window, becomes a
-tile of its own: the spanned window's otherwise empty slot starts at the graph's first row).  Checks on the C2 structure
-and on random partitions that the tiles stay a partition of [0, N), never exceed the stage, and that the +-1 window
-search of collect_cut_heavy finds the tile of every row; prints the share of rows left in cut tiles.
+collect_cut_heavy_kernel), no GPU: graphs longer than the window are cut -> checked slow path.  Checks on the C2
+structure and on random partitions that the tiles stay a partition of [0, N), never exceed the stage, and that the
+window search of collect_cut_heavy finds the tile of every row; prints the share of rows left in cut tiles.
 Usage: python tools/k1_tiles_model.py [window_rows]"""
 import os
 import sys
@@ -13,7 +11,7 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 
-def boundary(seg_ptr, C, N, k, T, whole):
+def boundary(seg_ptr, C, N, k, T):
     """(row, aligned) exactly as the device function computes it."""
     if k >= T:
         return N, True
@@ -22,27 +20,23 @@ def boundary(seg_ptr, C, N, k, T, whole):
     gs = int(seg_ptr[lo])
     if gs < target + C:
         return gs, True
-    if whole and lo >= 1:
-        s, e = int(seg_ptr[lo - 1]), gs                             # the graph that spans window k
-        if e - s <= 2 * C:
-            return (s if k == s // C + 1 else e), True
     return target, False
 
 
-def make_tiles(seg_ptr, C, whole):
+def make_tiles(seg_ptr, C):
     N = int(seg_ptr[-1])
     T = (N + C - 1) // C
     tiles = []
     for k in range(T):
-        r0, a0 = boundary(seg_ptr, C, N, k, T, whole)
-        r1, a1 = boundary(seg_ptr, C, N, k + 1, T, whole)
+        r0, a0 = boundary(seg_ptr, C, N, k, T)
+        r1, a1 = boundary(seg_ptr, C, N, k + 1, T)
         tiles.append((r0, r1, not (a0 and a1)))
     return tiles
 
 
-def check(seg_ptr, C, whole):
+def check(seg_ptr, C):
     N = int(seg_ptr[-1])
-    tiles = make_tiles(seg_ptr, C, whole)
+    tiles = make_tiles(seg_ptr, C)
     T = len(tiles)
     assert tiles[0][0] == 0 and tiles[-1][1] == N
     for (a0, a1, _), (b0, _, _) in zip(tiles[:-1], tiles[1:]):
@@ -52,40 +46,14 @@ def check(seg_ptr, C, whole):
         if not cut:
             assert r1 - r0 <= 2 * C, (r0, r1)
             assert r0 in starts and r1 in starts          # closed tiles hold whole graphs only
-    # the tile of every row, found as collect_cut_heavy_kernel does (window of the row, then one step left or right)
+    # the tile of every row, found as collect_cut_heavy_kernel does (window of the row, then one step left)
     x = np.array([t[0] for t in tiles]); y = np.array([t[1] for t in tiles])
     r = np.arange(N)
     k = np.minimum(r // C, T - 1)
     k = np.where(r < x[k], k - 1, k)
-    if whole:
-        k = np.where((r >= y[k]) & (k + 1 < T), k + 1, k)
     assert ((x[k] <= r) & (r < y[k])).all()
     cut_rows = sum(r1 - r0 for r0, r1, cut in tiles if cut)
     return cut_rows / max(N, 1), max((r1 - r0 for r0, r1, cut in tiles if not cut), default=0)
-
-
-def device_balance(desc, H, heavy_cost, G):
-    """the slot permutation balance_tiles_kernel (-DDN4GL_TILE_BALANCE) computes, restated: desc = [(r0, r1, e0, e1, cut)],
-    H listed long rows with costs heavy_cost dealt to CTAs i % G first; returns (dest, load): dest[k] = slot of the k-th
-    tile in cost order (ties: lower index first), load = estimated CTA loads afterwards."""
-    T = len(desc)
-    cost = [((e1 - e0) >> 2) + (r1 - r0) for r0, r1, e0, e1, _ in desc]
-    cost = [2 * c if d[4] else c for c, d in zip(cost, desc)]
-    order = sorted(range(T), key=lambda i: (-cost[i], i))
-    load = [0] * G
-    for i in range(H):
-        load[i % G] += heavy_cost[i]
-    first = [((b - H % G) % G + G) % G for b in range(G)]
-    free = [((T - 1 - f) // G + 1) if f < T else 0 for f in first]
-    used = [0] * G
-    dest = []
-    for i in order:
-        b = min((load[b], b) for b in range(G) if free[b] > 0)[1]
-        dest.append(first[b] + used[b] * G)
-        used[b] += 1
-        free[b] -= 1
-        load[b] += cost[i]
-    return order, dest, load
 
 
 def main():
@@ -96,58 +64,14 @@ def main():
         if trial % 3 == 0:
             n = np.minimum(n, int(rng.integers(1, 2 * C + 2)))
         seg = np.concatenate([[0], np.cumsum(n)])
-        for whole in (False, True):
-            check(seg, C, whole)
+        check(seg, C)
     from dummynode4graphlearning_b200 import synth
     from oracle import transforms as OT   # dev tool: the oracle builds the C2 structure on the host
     conj = OT.tu_conjugate(OT.tu_add_dummy(synth.tu_batch("proteins", 1113, seed=0)))
     seg = conj["node_ptr"].astype(np.int64)
-    s_, d_, _, _ = OT.pyg_coalesce(conj["src"], conj["dst"])
-    deg = np.bincount(d_, minlength=int(seg[-1]))
-    row_cost = deg // 4 + deg % 4 + 1                     # four-neighbour batches + remainders + row overhead
-    for whole in (False, True):
-        share, biggest = check(seg, C, whole)
-        print("C2, window %d, %s: %.1f %% of the rows in cut tiles (checked slow path), largest closed tile %d rows"
-              % (C, "whole graphs up to 2 windows" if whole else "shipped rule", 100 * share, biggest))
-        # round-robin deal of the work items over 148 persistent CTAs (long rows of cut tiles first, as the kernel does);
-        # rows on the checked path are charged SLOW x the unchecked cost (an assumption -- the timeline only says "slower")
-        for slow in (1.5, 2.5):
-            items = []
-            tiles = make_tiles(seg, C, whole)
-            for r0, r1, cut in tiles:
-                if cut:
-                    items += [float(np.ceil(deg[r] / 31.0 / 4.0) + 8) for r in range(r0, r1) if deg[r] > 64]
-            for r0, r1, cut in tiles:
-                c = row_cost[r0:r1]
-                if cut:
-                    c = np.where(deg[r0:r1] > 64, 0, c)
-                items.append(float(c.sum()) * (slow if cut else 1.0) / 31.0)
-            def deal(seq, serpentine=False):
-                load = np.zeros(148)
-                for i, w in enumerate(seq):
-                    r, c = divmod(i, 148)
-                    load[147 - c if (serpentine and r % 2) else c] += w
-                return load.max() / load.mean()
-            H = len(items) - len(tiles)
-            by_cost = items[:H] + sorted(items[H:], reverse=True)       # long rows first as today, then tiles by cost
-            lpt = np.zeros(148)
-            for w in sorted(items, reverse=True):
-                lpt[lpt.argmin()] += w
-            # greedy longest-first under the round-robin deal's fixed slot counts (a pure permutation of the tile slots:
-            # CTA b owns the slots i with (H + i) % 148 == b; the long rows stay where they are)
-            T = len(tiles)
-            load = np.zeros(148)
-            for i in range(H):
-                load[i % 148] += items[i]
-            free = np.bincount((H + np.arange(T)) % 148, minlength=148)
-            for w in sorted(items[H:], reverse=True):
-                b = int(np.where(free > 0, load, np.inf).argmin())
-                load[b] += w
-                free[b] -= 1
-            print("    checked path %.1fx: %d items, max / mean CTA load: as dealt today %.2f, tiles sorted by cost %.2f, "
-                  "sorted + serpentine %.2f, greedy longest-first %.2f, the same as a permutation of the tile slots %.2f"
-                  % (slow, len(items), deal(items), deal(by_cost), deal(by_cost, True), lpt.max() / lpt.mean(),
-                     load.max() / load.mean()))
+    share, biggest = check(seg, C)
+    print("C2, window %d: %.1f %% of the rows in cut tiles (checked slow path), largest closed tile %d rows"
+          % (C, 100 * share, biggest))
 
 
 if __name__ == "__main__":

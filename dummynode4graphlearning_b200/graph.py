@@ -66,6 +66,18 @@ class CSR:
         self.block_diagonal = False   # True: built graph by graph over seg_ptr (the tiling skips its column verification)
         self._tiles = {}
 
+    def clone(self, seg_ptr, *, eid, tiles):
+        """private copy of the device arrays over the row offsets `seg_ptr` (the buffers a captured CUDA graph reads);
+        the edge ids and the cached tilings are copied only when asked for (else None / empty)."""
+        c = CSR(self.row_ptr.clone(), self.col.clone(), self.eid.clone() if eid else None, self.n_rows, self.nnz)
+        c.heavy_rows = None if self.heavy_rows is None else self.heavy_rows.clone()
+        c.heavy_count = None if self.heavy_count is None else self.heavy_count.clone()
+        c.heavy_thr, c.seg_ptr, c.max_seg, c.block_diagonal = self.heavy_thr, seg_ptr, self.max_seg, self.block_diagonal
+        if tiles:
+            c._tiles = {key: {k: (v.clone() if isinstance(v, torch.Tensor) else v) for k, v in t.items()}
+                        for key, t in self._tiles.items()}
+        return c
+
     def tiles(self, D, smem_bytes=None):
         """tiling + launch configuration of the pipelined aggregation kernel for feature width D (cached).
 

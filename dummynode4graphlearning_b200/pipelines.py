@@ -16,7 +16,7 @@ import torch.nn.functional as F
 
 from . import ops
 from . import transforms as T
-from .graph import CSR, BatchedGraph
+from .graph import BatchedGraph
 from .graph_classification.data import Batch
 from .parallel import GradientBucket, is_distributed, sync_padded_lengths
 
@@ -62,14 +62,14 @@ def _structure_tensors(data):
     return tensors, scalars
 
 
-def _signature(data):
-    tensors, scalars = _structure_tensors(data)
+def _signature(tensors, scalars):
+    """CUDA-graph signature of a train step from the tensors it reads and the host scalars baked into its launches."""
     return (tuple(None if t is None else (tuple(t.shape), t.dtype) for t in tensors), tuple(scalars))
 
 
 def _static_clone(data):
     """a Batch with the same compiled structure whose tensors are private copies (the buffers a captured CUDA graph
-    reads); returns (batch, tensor list in _structure_tensors order)."""
+    reads).  The tilings are copied: the captured forward reads them as they are (_structure_tensors lists them)."""
     import copy
     s0 = data.structure
     d = Batch(data.x.clone(), None, None, y=data.y.clone())
@@ -78,24 +78,9 @@ def _static_clone(data):
     s._row2seg = None if s0.row2seg is None else s0.row2seg.clone()
     s._rel = {}
     for name in ("csr_in", "csr_out"):
-        c0 = getattr(s0, name)
-        c = CSR(c0.row_ptr.clone(), c0.col.clone(), None, c0.n_rows, c0.nnz)
-        c.heavy_rows = None if c0.heavy_rows is None else c0.heavy_rows.clone()
-        c.heavy_count = None if c0.heavy_count is None else c0.heavy_count.clone()
-        c.heavy_thr, c.seg_ptr, c.max_seg, c.block_diagonal = c0.heavy_thr, s.node_ptr, c0.max_seg, c0.block_diagonal
-        for key, t in c0._tiles.items():
-            c._tiles[key] = {k: (v.clone() if isinstance(v, torch.Tensor) else v) for k, v in t.items()}
-        setattr(s, name, c)
+        setattr(s, name, getattr(s0, name).clone(s.node_ptr, eid=False, tiles=True))
     d._structure = s
-    return d, _structure_tensors(d)[0]
-
-
-def _batch_tensors(data):
-    """every device tensor a compiled Batch holds (what the train step may read from it)."""
-    s = data.structure
-    out = [t for t in _structure_tensors(data)[0] if t is not None]
-    out += [t for t in (s.src, s.dst, s.csr_in.eid, s.csr_out.eid) if t is not None]
-    return out
+    return d
 
 
 class PendingLoss:
@@ -132,36 +117,44 @@ class PendingLoss:
         return self.value
 
 
-class _CapturedStep:
-    """one CUDA graph of (forward, loss, backward, gradient all-reduce, optimizer step) for ONE batch signature.
-    Replaying it does all of that work again on the data currently held by the static buffers."""
+class _CapturedGraph:
+    """one CUDA graph of ``fn()``, captured on `stream` (default: torch's own capture stream).  ``replay()`` does the
+    captured work again and returns what ``fn()`` returned during the capture (static tensors)."""
 
-    def __init__(self, pipe, data):
-        self.batch, self.static = _static_clone(data)
-        self.replays = 0
-        self.graph = torch.cuda.CUDAGraph()
-        torch.cuda.synchronize()
+    def __init__(self, fn, stream=None):
         from ._lib import lib
+        self.graph, self.replays = torch.cuda.CUDAGraph(), 0
         k0 = lib().kernel_launches()
+        with torch.cuda.graph(self.graph, stream=stream):
+            self.out = fn()
+        self.library_kernels = lib().kernel_launches() - k0   # libdn4gl kernels inside the graph (launched per replay)
+
+    def replay(self):
+        self.graph.replay()
+        self.replays += 1
+        return self.out
+
+
+class _CapturedStep(_CapturedGraph):
+    """one train step (forward, loss, backward, gradient all-reduce, optimizer step) for ONE batch signature, captured as
+    ``body(*batch)`` on `batch`, a private copy of a batch whose tensors ``describe(*batch)`` lists.  ``load()`` of
+    another batch of the signature followed by ``replay()`` does all of that work again on that batch's data."""
+
+    def __init__(self, body, batch, describe):
+        self.batch, self.static = batch, describe(*batch)[0]
+        torch.cuda.synchronize()
         # the AccumulateGrad nodes were created by the eager steps on the default stream; capture runs them on the
         # capture stream, which is intended here
         torch.autograd.graph.set_warn_on_accumulate_grad_stream_mismatch(False)
-        with torch.cuda.graph(self.graph):
-            self.loss = pipe._train_body(self.batch)
-        self.library_kernels = lib().kernel_launches() - k0   # libdn4gl kernels inside the graph (launched per replay)
+        super().__init__(lambda: body(*batch))
 
-    def run(self, data):
-        src = _structure_tensors(data)[0]
-        pairs = [(d, s) for d, s in zip(self.static, src) if d is not None]
+    def load(self, tensors):
+        """copies a batch's tensors (in ``describe`` order) into the buffers the graph reads."""
+        pairs = [(d, s) for d, s in zip(self.static, tensors) if d is not None]
         torch._foreach_copy_([d for d, _ in pairs], [s for _, s in pairs])
-        self.copied = torch.cuda.Event()     # from here on the batch's own tensors may be overwritten (captured transform)
-        self.copied.record()
-        self.graph.replay()
-        self.replays += 1
-        return self.loss
 
 
-class _CapturedTransform:
+class _CapturedTransform(_CapturedGraph):
     """CUDA graph of the whole transform (dummy augmentation, edge-to-vertex transform, canonicalisation, both CSR builds,
     tilings) for ONE raw-batch signature.  Only possible when the transform has no device->host read, i.e. when the
     loader attached ``conj_sizes`` (transforms.tu_conjugate_sizes).  The ~60 small launches that the eager transform paces
@@ -169,16 +162,11 @@ class _CapturedTransform:
     must not start before the train step that consumes the previous outputs has copied them (``wait`` event)."""
 
     def __init__(self, pipe, dev_batch):
-        self.static_in = {k: (v.clone() if isinstance(v, torch.Tensor) else v) for k, v in dev_batch.items()}
-        self.graph = torch.cuda.CUDAGraph()
-        from ._lib import lib
-        k0 = lib().kernel_launches()
         cur = torch.cuda.current_stream()
+        cur.synchronize()
+        self.static_in = {k: (v.clone() if isinstance(v, torch.Tensor) else v) for k, v in dev_batch.items()}
         on_side = cur != torch.cuda.default_stream(cur.device)      # capture must not run on the legacy default stream
-        with torch.cuda.graph(self.graph, **({"stream": cur} if on_side else {})):
-            self.out = pipe._transform_eager(self.static_in)
-        self.library_kernels = lib().kernel_launches() - k0
-        self.replays = 0
+        super().__init__(lambda: pipe._transform_eager(self.static_in), stream=cur if on_side else None)
 
     def run(self, batch, wait=None):
         """batch: device OR pinned-host tensors of the captured signature (copied into the graph's input buffers)."""
@@ -188,9 +176,7 @@ class _CapturedTransform:
             if isinstance(v, torch.Tensor):
                 d = self.static_in[k]
                 d.copy_(v if v.dtype == d.dtype else v.to(d.dtype), non_blocking=True)
-        self.graph.replay()
-        self.replays += 1
-        return self.out
+        return self.replay()
 
 
 def _raw_signature(b):
@@ -198,7 +184,92 @@ def _raw_signature(b):
                          (tuple(v) if isinstance(v, (tuple, list)) else v)) for k, v in b.items()))
 
 
-class ClassificationPipeline:
+class _Pipeline:
+    """what both pipelines share: the CUDA-graph cache of the train step and the overlapped step, whose transform runs on
+    a second stream while the previous train step still runs on the current one."""
+
+    _caches = ("_graphs",)      # attributes that hold captured graphs by signature
+
+    def __init__(self, model, optimizer, cuda_graphs, max_graphs, overlap):
+        self.model, self.opt = model, optimizer
+        self.bucket = getattr(optimizer, "bucket", None) or GradientBucket(model.parameters())
+        self.device = next(model.parameters()).device
+        self.global_batch = None
+        capturable = all(g.get("capturable", False) for g in optimizer.param_groups)
+        self.cuda_graphs = capturable if cuda_graphs is None else bool(cuda_graphs)
+        if self.cuda_graphs and not capturable:
+            raise ValueError("cuda_graphs=True needs an optimizer built with capturable=True")
+        self._graphs, self._max_graphs = {}, max_graphs     # captured train steps by batch signature
+        self.overlap = bool(self.cuda_graphs if overlap is None else overlap) and self.device.type == "cuda"
+        self._tstream = None
+        self._inflight = []      # completion events of the train steps queued so far (bounded lead, see _throttle)
+
+    def _captured(self, cache, sig, capture):
+        """the CUDA graph to replay for a batch of signature `sig`, or None when the batch runs eagerly.  The first
+        occurrence of a signature runs eagerly and is remembered as "seen" (while `cache` holds fewer than max_graphs
+        signatures), the second is captured by ``capture()``, later ones replay that graph."""
+        ent = cache.get(sig)
+        if ent is None:
+            if len(cache) < self._max_graphs:
+                cache[sig] = "seen"
+        elif isinstance(ent, str):
+            ent = cache[sig] = capture()
+        return ent
+
+    def replayed_library_kernels(self):
+        """libdn4gl kernels launched through CUDA-graph replays so far (they bypass the library's launch counter)."""
+        return sum(e.replays * e.library_kernels for name in self._caches for e in getattr(self, name).values()
+                   if isinstance(e, _CapturedGraph))
+
+    def _transform_stream(self):
+        if self._tstream is None:
+            # high priority: the host blocks on the transform's two size read-backs, so its small kernels should be
+            # scheduled ahead of the queued CTAs of the train step that runs concurrently on the main stream
+            self._tstream = torch.cuda.Stream(self.device, priority=-1)
+        return self._tstream
+
+    def _throttle(self):
+        """bounds the host's lead over the train stream to ONE step: before the transform of step k+1 starts, the train
+        step k-1 must have finished (step k may still be running -- that is the overlap).  Without the bound the host
+        (whose transform only synchronises with its own stream) runs several steps ahead whenever the train stream is
+        the slower side; every step in flight pins a full set of transform outputs, the caching allocator answers with
+        cudaMalloc, and single steps stall for 5-50 ms (profiles/r1f)."""
+        while len(self._inflight) >= 2:
+            self._inflight.pop(0).synchronize()
+
+    def _mark_step(self):
+        ev = torch.cuda.Event()
+        ev.record()
+        self._inflight.append(ev)
+
+    def _hand_over(self, tensors, tstream):
+        """transform outputs (`tensors`, allocated and produced on `tstream`) -> consumable on the current (train) stream."""
+        main = torch.cuda.current_stream()
+        done = torch.cuda.Event()
+        done.record(tstream)
+        main.wait_event(done)
+        for t in tensors:       # the caching allocator must not recycle them before the train stream is done
+            t.record_stream(main)
+
+    def _step_overlapped(self, transform, train, assume_ready):
+        """``train(transform())`` with the transform on the second stream (see ClassificationPipeline.step_resident);
+        ``_transform_outputs`` names the tensors of its result that the train stream takes over."""
+        ts = self._transform_stream()
+        self._throttle()
+        if not assume_ready:
+            ts.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(ts):
+            out = transform()
+            tensors = self._transform_outputs(out)
+        self._hand_over(tensors, ts)
+        loss = train(out)
+        self._mark_step()
+        return loss
+
+
+class ClassificationPipeline(_Pipeline):
+    _caches = ("_graphs", "_tgraphs")
+
     def __init__(self, model, optimizer, mode="conj", num_node_labels=None, num_edge_labels=None,
                  node_label_min=None, with_edge_attr=False, cuda_graphs=None, max_graphs=8, overlap=None):
         """mode: 'dummy' (DUMMY_ graphs), 'conj' (CONJ_: dummy + edge-to-vertex), 'line' (LINE_), 'raw'.
@@ -213,29 +284,12 @@ class ClassificationPipeline:
         signature runs eagerly, the second is captured, later ones are replayed (a ~300-launch step is host-bound
         otherwise, profiles/).  Needs an optimizer whose step is capturable (``torch.optim.Adam(capturable=True)``);
         default: on exactly when the optimizer is."""
-        self.model, self.opt, self.mode = model, optimizer, mode
+        super().__init__(model, optimizer, cuda_graphs, max_graphs, overlap)
+        self.mode = mode
         self.nvl, self.nel = num_node_labels, num_edge_labels
         self.node_label_min, self.with_edge_attr = node_label_min, with_edge_attr
-        self.bucket = getattr(optimizer, "bucket", None) or GradientBucket(model.parameters())
-        self.device = next(model.parameters()).device
-        self.global_batch = None
-        capturable = all(g.get("capturable", False) for g in optimizer.param_groups)
-        self.cuda_graphs = capturable if cuda_graphs is None else bool(cuda_graphs)
-        if self.cuda_graphs and not capturable:
-            raise ValueError("cuda_graphs=True needs an optimizer built with capturable=True")
-        self._graphs, self._max_graphs = {}, max_graphs
         self._tgraphs = {}       # captured transforms by raw-batch signature
         self._consumed = None    # event: the latest train step no longer reads its batch's own tensors
-        self.overlap = bool(self.cuda_graphs if overlap is None else overlap) and self.device.type == "cuda"
-        self._tstream = None
-        self._inflight = []      # completion events of the train steps queued so far (bounded lead, see _throttle)
-
-    def _transform_stream(self):
-        if self._tstream is None:
-            # high priority: the host blocks on the transform's two size read-backs, so its small kernels should be
-            # scheduled ahead of the queued CTAs of the train step that runs concurrently on the main stream
-            self._tstream = torch.cuda.Stream(self.device, priority=-1)
-        return self._tstream
 
     def transform(self, batch):
         """raw TU-shaped batch (device tensors, or pinned host tensors of an int32 / float32 / int64-y batch) -> PyG-style
@@ -248,16 +302,9 @@ class ClassificationPipeline:
         if capturable:
             norm = {k: (v.to(torch.int32) if isinstance(v, torch.Tensor) and v.dtype == torch.int64 and k != "y" else v)
                     for k, v in batch.items()} if on_host else batch
-            sig = _raw_signature(norm)
-            ent = self._tgraphs.get(sig)
-            if ent is None:
-                if len(self._tgraphs) < self._max_graphs:
-                    self._tgraphs[sig] = "seen"
-            else:
-                if ent == "seen":
-                    dev_b = self._upload(batch) if on_host else batch
-                    torch.cuda.current_stream().synchronize()
-                    ent = self._tgraphs[sig] = _CapturedTransform(self, dev_b)
+            ent = self._captured(self._tgraphs, _raw_signature(norm),
+                                 lambda: _CapturedTransform(self, self._upload(batch) if on_host else batch))
+            if ent is not None:
                 # the outputs are static tensors: the consumer of the previous replay must be done with them -- a replayed
                 # train step right after its copy into its own buffers, an eager one at its end (train_on sets the event)
                 return ent.run(norm, wait=self._consumed)
@@ -310,54 +357,30 @@ class ClassificationPipeline:
         # bound to the stream they were created on) alive into the next step / a CUDA-graph capture
         return loss.detach()
 
-    def replayed_library_kernels(self):
-        """libdn4gl kernels launched through CUDA-graph replays so far (they bypass the library's launch counter)."""
-        return (sum(e.replays * e.library_kernels for e in self._graphs.values() if isinstance(e, _CapturedStep)) +
-                sum(e.replays * e.library_kernels for e in self._tgraphs.values() if isinstance(e, _CapturedTransform)))
-
     def train_on(self, data):
         if not self.model.training:      # Module.train() walks every submodule (~0.2 ms of host time per step)
             self.model.train()
         if not self.cuda_graphs:
             return self._train_body(data)
-        sig = _signature(data)
-        ent = self._graphs.get(sig)
-        if ent is None:                                     # first time this signature is seen: a normal eager step
-            if len(self._graphs) < self._max_graphs:
-                self._graphs[sig] = "seen"
+        tensors, scalars = _structure_tensors(data)
+        ent = self._captured(self._graphs, _signature(tensors, scalars),
+                             lambda: _CapturedStep(self._train_body, (_static_clone(data),), _structure_tensors))
+        if ent is None:
             loss = self._train_body(data)
-            self._consumed = torch.cuda.Event()
-            self._consumed.record()
-            return loss
-        if ent == "seen":
-            ent = self._graphs[sig] = _CapturedStep(self, data)
-        loss = ent.run(data)
-        self._consumed = ent.copied
-        return loss
+        else:
+            ent.load(tensors)
+        # from here on the batch's own tensors may be overwritten (captured transform): after an eager step's end, right
+        # after a replay's copy into the graph's buffers
+        self._consumed = torch.cuda.Event()
+        self._consumed.record()
+        return loss if ent is None else ent.replay()
 
-    def _throttle(self):
-        """bounds the host's lead over the train stream to ONE step: before the transform of step k+1 starts, the train
-        step k-1 must have finished (step k may still be running -- that is the overlap).  Without the bound the host
-        (whose transform only synchronises with its own stream) runs several steps ahead whenever the train stream is
-        the slower side; every step in flight pins a full set of transform outputs, the caching allocator answers with
-        cudaMalloc, and single steps stall for 5-50 ms (profiles/r1f)."""
-        while len(self._inflight) >= 2:
-            self._inflight.pop(0).synchronize()
-
-    def _mark_step(self):
-        ev = torch.cuda.Event()
-        ev.record()
-        self._inflight.append(ev)
-
-    def _hand_over(self, data, tstream):
-        """transform output (allocated and produced on `tstream`) -> consumable on the current (train) stream."""
-        main = torch.cuda.current_stream()
-        done = torch.cuda.Event()
-        done.record(tstream)
-        main.wait_event(done)
-        for t in _batch_tensors(data):       # the caching allocator must not recycle them before the train stream is done
-            t.record_stream(main)
-        return data
+    def _transform_outputs(self, data):
+        """every device tensor a compiled Batch holds (what the train step may read from it)."""
+        s = data.structure
+        out = [t for t in _structure_tensors(data)[0] if t is not None]
+        out += [t for t in (s.src, s.dst, s.csr_in.eid, s.csr_out.eid) if t is not None]
+        return out
 
     def step_resident(self, dev_batch, assume_ready=False):
         """inputs already in HBM: transform + train step; returns the loss tensor (no host sync).
@@ -368,15 +391,7 @@ class ClassificationPipeline:
         queued on the current stream so far (always safe, no GPU-side overlap)."""
         if not self.overlap:
             return self.train_on(self.transform(dev_batch))
-        ts = self._transform_stream()
-        self._throttle()
-        if not assume_ready:
-            ts.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(ts):
-            data = self.transform(dev_batch)
-        loss = self.train_on(self._hand_over(data, ts))
-        self._mark_step()
-        return loss
+        return self._step_overlapped(lambda: self.transform(dev_batch), self.train_on, assume_ready)
 
     def _upload(self, host_batch):
         dev = upload(host_batch, self.device)
@@ -389,13 +404,8 @@ class ClassificationPipeline:
         loop that reads the previous step's result after submitting the next one keeps both streams busy."""
         if not self.overlap:
             return PendingLoss(self.step_resident(self._upload(host_batch)))
-        ts = self._transform_stream()
-        self._throttle()
-        with torch.cuda.stream(ts):          # the upload is ordered on the transform stream: no wait on the train stream
-            data = self.transform(host_batch)
-        loss = self.train_on(self._hand_over(data, ts))
-        self._mark_step()
-        return PendingLoss(loss)
+        # the upload is ordered on the transform stream: no wait on the train stream
+        return PendingLoss(self._step_overlapped(lambda: self.transform(host_batch), self.train_on, assume_ready=True))
 
     def step(self, host_batch):
         """host buffers in, python float out: H2D + transform + train step + D2H of the loss (blocking)."""
@@ -422,50 +432,29 @@ def _graph_tensors(g):
     return tensors, scalars
 
 
+def _counting_tensors(pattern, graph, counts):
+    """every device tensor a counting train step reads (fixed order) + the host scalars of its CUDA-graph signature."""
+    tp, sp = _graph_tensors(pattern)
+    tg, sg = _graph_tensors(graph)
+    return tp + tg + [counts], [tuple(sp), tuple(sg)]
+
+
 def _static_graph(g):
     """private copy of a BatchedGraph (the buffers a captured CUDA graph reads); caches that the model fills during its
-    forward (relation CSRs, int32 views, tilings) start empty so that the captured forward recomputes them."""
+    forward (relation CSRs, int32 views, tilings) start empty so that the captured forward recomputes them.  Tilings
+    copied from this batch would not be among the tensors a replay copies in (_graph_tensors), so later replays would
+    run on this batch's tiles."""
     c = BatchedGraph(g.src.clone(), g.dst.clone(), g.node_ptr.clone(), g.edge_ptr.clone(),
                      {k: v.clone() for k, v in g.ndata.items()}, {k: v.clone() for k, v in g.edata.items()})
     c._n, c._host_sizes, c._pad_lengths = g._n, g._host_sizes, g._pad_lengths
     for name in ("_csr_in", "_csr_out"):
         c0 = getattr(g, name)
         if c0 is not None:
-            n = CSR(c0.row_ptr.clone(), c0.col.clone(), c0.eid.clone(), c0.n_rows, c0.nnz)
-            n.heavy_rows = None if c0.heavy_rows is None else c0.heavy_rows.clone()
-            n.heavy_count = None if c0.heavy_count is None else c0.heavy_count.clone()
-            n.heavy_thr, n.seg_ptr, n.max_seg = c0.heavy_thr, c.node_ptr, c0.max_seg
-            setattr(c, name, n)
+            setattr(c, name, c0.clone(c.node_ptr, eid=True, tiles=False))
     return c
 
 
-class _CapturedCountingStep:
-    """CUDA graph of one counting train step (forward, loss, backward, all-reduce, clipping, optimizer) for one
-    (pattern, graph) batch signature."""
-
-    def __init__(self, pipe, pattern, graph, counts):
-        from ._lib import lib
-        self.pattern, self.graph_batch, self.counts = _static_graph(pattern), _static_graph(graph), counts.clone()
-        self.static = _graph_tensors(self.pattern)[0] + _graph_tensors(self.graph_batch)[0] + [self.counts]
-        self.replays = 0
-        self.graph = torch.cuda.CUDAGraph()
-        torch.cuda.synchronize()
-        k0 = lib().kernel_launches()
-        torch.autograd.graph.set_warn_on_accumulate_grad_stream_mismatch(False)
-        with torch.cuda.graph(self.graph):
-            self.loss = pipe._train_body(self.pattern, self.graph_batch, self.counts)
-        self.library_kernels = lib().kernel_launches() - k0
-
-    def run(self, pattern, graph, counts):
-        src = _graph_tensors(pattern)[0] + _graph_tensors(graph)[0] + [counts]
-        pairs = [(d, s) for d, s in zip(self.static, src) if d is not None]
-        torch._foreach_copy_([d for d, _ in pairs], [s for _, s in pairs])
-        self.graph.replay()
-        self.replays += 1
-        return self.loss
-
-
-class CountingPipeline:
+class CountingPipeline(_Pipeline):
     def __init__(self, model, optimizer, config, add_dummy=True, rep_reg_w=0.0, neg_slp=0.01, max_grad_norm=8.0,
                  cuda_graphs=None, max_graphs=8, overlap=None, exact_sharding=False, bp_loss="MSE", match_loss_w=0.0,
                  match_reg_w=0.0, remove_loops=False, add_rev=False, convert_conj=False, share_emb_net=True):
@@ -481,8 +470,8 @@ class CountingPipeline:
         data-set level preprocessing switches, applied per mini-batch on the GPU in the reference's order
         (train.py:1271-1340: loops, reversed edges, dummy, edge-to-vertex), each with the maxima the previous steps
         leave behind; build the model with ``transforms.process_model_config`` of the same switches."""
-        self.model, self.opt, self.cfg, self.add_dummy = model, optimizer, config, add_dummy
-        self.device = next(model.parameters()).device
+        super().__init__(model, optimizer, cuda_graphs, max_graphs, overlap)
+        self.cfg, self.add_dummy = config, add_dummy
         # neg_slp and rep_reg_w change every step in the reference (train.py:648-740 recomputes them from their
         # schedules): they live in device scalars that the (possibly captured) train step READS, so an update through the
         # properties below is seen by the next step / CUDA-graph replay
@@ -491,22 +480,9 @@ class CountingPipeline:
         self._neg_slp = self._rep_reg_w = None
         self.neg_slp, self.rep_reg_w, self.max_grad_norm = neg_slp, rep_reg_w, max_grad_norm
         self.share_emb_net = bool(share_emb_net)
-        self.bucket = getattr(optimizer, "bucket", None) or GradientBucket(model.parameters())
-        self.global_batch = None
-        capturable = all(g.get("capturable", False) for g in optimizer.param_groups)
-        self.cuda_graphs = capturable if cuda_graphs is None else bool(cuda_graphs)
-        if self.cuda_graphs and not capturable:
-            raise ValueError("cuda_graphs=True needs an optimizer built with capturable=True")
-        self._graphs, self._max_graphs = {}, max_graphs
-        self.overlap = bool(self.cuda_graphs if overlap is None else overlap) and self.device.type == "cuda"
-        self._tstream, self._inflight = None, []
         self.exact_sharding = bool(exact_sharding)
         self.bp_loss, self.match_loss_w, self.match_reg_w = bp_loss, match_loss_w, match_reg_w
         self.remove_loops, self.add_rev, self.convert_conj = bool(remove_loops), bool(add_rev), bool(convert_conj)
-
-    _transform_stream = ClassificationPipeline._transform_stream
-    _throttle = ClassificationPipeline._throttle
-    _mark_step = ClassificationPipeline._mark_step
 
     @property
     def neg_slp(self):
@@ -603,9 +579,6 @@ class CountingPipeline:
         self.opt.step()
         return loss.detach()   # see ClassificationPipeline._train_body
 
-    def replayed_library_kernels(self):
-        return sum(e.replays * e.library_kernels for e in self._graphs.values() if isinstance(e, _CapturedCountingStep))
-
     def train_on(self, pattern, graph, counts, node_weights=None, edge_weights=None):
         if not self.model.training:      # Module.train() walks every submodule (~0.2 ms of host time per step)
             self.model.train()
@@ -613,43 +586,28 @@ class CountingPipeline:
             return self._train_body(pattern, graph, counts, node_weights, edge_weights)
         if not self.cuda_graphs:
             return self._train_body(pattern, graph, counts)
-        tp, sp = _graph_tensors(pattern)
-        tg, sg = _graph_tensors(graph)
-        sig = (tuple(None if t is None else (tuple(t.shape), t.dtype) for t in tp + tg), tuple(sp), tuple(sg),
-               tuple(counts.shape))
-        ent = self._graphs.get(sig)
+        tensors, scalars = _counting_tensors(pattern, graph, counts)
+        ent = self._captured(self._graphs, _signature(tensors, scalars), lambda: _CapturedStep(
+            self._train_body, (_static_graph(pattern), _static_graph(graph), counts.clone()), _counting_tensors))
         if ent is None:
-            if len(self._graphs) < self._max_graphs:
-                self._graphs[sig] = "seen"
             return self._train_body(pattern, graph, counts)
-        if ent == "seen":
-            ent = self._graphs[sig] = _CapturedCountingStep(self, pattern, graph, counts)
-        return ent.run(pattern, graph, counts)
+        ent.load(tensors)
+        return ent.replay()
+
+    def _transform_outputs(self, graphs):
+        """every device tensor of both graphs; everything the captured step copies out of the batch exists before the
+        hand-over (the CSRs are built here, on the transform's stream, if the transform left one out)."""
+        for g in graphs:
+            g.csr_in, g.csr_out
+        return [t for g in graphs for t in _graph_tensors(g)[0] if t is not None]
 
     def step_resident(self, p_dev, g_dev, counts_dev, assume_ready=False):
         """see ClassificationPipeline.step_resident: with ``overlap`` the augmentation + CSR builds of this mini-batch run
         on the second stream while the previous train step is still executing."""
         if not self.overlap:
-            pattern, graph = self.transform(p_dev, g_dev)
-            return self.train_on(pattern, graph, counts_dev)
-        main = torch.cuda.current_stream()
-        ts = self._transform_stream()
-        self._throttle()
-        if not assume_ready:
-            ts.wait_stream(main)
-        with torch.cuda.stream(ts):
-            pattern, graph = self.transform(p_dev, g_dev)
-            for g in (pattern, graph):       # everything the captured step copies out of the batch exists before the hand-over
-                g.csr_in, g.csr_out
-        done = torch.cuda.Event()
-        done.record(ts)
-        main.wait_event(done)
-        for t in _graph_tensors(pattern)[0] + _graph_tensors(graph)[0]:
-            if t is not None:
-                t.record_stream(main)
-        loss = self.train_on(pattern, graph, counts_dev)
-        self._mark_step()
-        return loss
+            return self.train_on(*self.transform(p_dev, g_dev), counts_dev)
+        return self._step_overlapped(lambda: self.transform(p_dev, g_dev),
+                                     lambda graphs: self.train_on(*graphs, counts_dev), assume_ready)
 
     def step(self, p_host, g_host, counts_host):
         p_dev, g_dev = upload(p_host, self.device), upload(g_host, self.device)

@@ -651,6 +651,8 @@ def dot(a, b, out=None, counter_slot=0):
     L = lib()
     if out is None:
         out = torch.empty(1, dtype=torch.float32, device=a.device)
+    if a.numel() == 0:      # an empty CUDA tensor has no storage (data_ptr() == 0), and its sum is 0: nothing to launch
+        return out.zero_()
     wsb = L.size("dn4gl_dot_workspace_bytes", a.numel())
     ws, counter = _tc_ws(a.device, wsb)
     L.call("dn4gl_dot_f32", ptr(a), ptr(b), a.numel(), ptr(out), ptr(ws), wsb, counter.data_ptr() + 4 * counter_slot, _stream())

@@ -434,7 +434,8 @@ size_t dn4gl_lin_workspace_bytes(int64_t N, int32_t K, int32_t M);
  * If bn_out != NULL the per-channel batch statistics of Y (biased variance, eps) are reduced in a fixed order and
  * the record {mean, rstd, gamma*rstd, beta} (gamma / beta NULL = 1 / 0) is written to bn_out[4*M]; running_mean /
  * running_var (momentum, unbiased variance) and num_batches_tracked are updated in place when non-NULL -- the
- * training-mode semantics of nn.BatchNorm1d.  ws: dn4gl_lin_workspace_bytes.  counters: DN4GL_LIN_COUNTERS int32 that are
+ * training-mode semantics of nn.BatchNorm1d (at N = 1, which nn.BatchNorm1d refuses in training, running_var takes the
+ * biased variance, 0).  ws: dn4gl_lin_workspace_bytes.  counters: DN4GL_LIN_COUNTERS int32 that are
  * 0 on entry and left 0 (arrival / ticket counters of the grid rendezvous that merges the per-CTA partials -- the stage
  * kernels are launched cooperatively; one array per stream that runs these stages concurrently).                      */
 int dn4gl_lin_fwd_f32(const float *X, int64_t N, int32_t K, const float *in_bn, int32_t in_act, float in_slope,

@@ -912,3 +912,32 @@ def gin_mlp_fusable(seq):
     if l1.bias is None or l2.bias is None:
         return False
     return lin_supported(l1.in_features, l1.out_features) and lin_supported(l2.in_features, l2.out_features)
+
+
+GATHER_MAX_COLUMNS = 8
+
+
+def gather_segments(idx, ptr_in, ptr_out, cols_in, cols_out, rebase=None, rebase_in=None, rebase_out=None):
+    """one level of a mini-batch assembled from a resident data set (dn4gl_gather_segments, one launch): segment
+    ``idx[k]`` of every column of ``cols_in`` (items ``ptr_in[idx[k]] ..``) lands at item ``ptr_out[k]`` of the matching
+    column of ``cols_out``; columns flagged in ``rebase`` (int32) also get ``rebase_out[k] - rebase_in[idx[k]]`` added.
+    idx / ptr_in / ptr_out / rebase_*: int32 device tensors; columns: contiguous device tensors of 4- or 8-byte items
+    whose leading dimension is the item count.  The caller checks that idx lies in the data set (datasets.py does)."""
+    import ctypes
+    import math
+    n = len(cols_in)
+    if n != len(cols_out) or not 1 <= n <= GATHER_MAX_COLUMNS:
+        raise ValueError("gather_segments: 1..%d input columns and as many outputs" % GATHER_MAX_COLUMNS)
+    words = []
+    for a, b in zip(cols_in, cols_out):
+        if (not (a.is_contiguous() and b.is_contiguous()) or a.dtype != b.dtype or a.shape[1:] != b.shape[1:]
+                or a.element_size() not in (4, 8)):
+            raise ValueError("gather_segments: columns must be contiguous, of 4- or 8-byte items, with matching dtype "
+                             "and item shape")
+        words.append(math.prod(a.shape[1:]) * a.element_size() // 4)
+    if cols_out[0].numel() == 0:        # the selected segments hold no items on this level
+        return
+    reb = [int(bool(r)) for r in (rebase or [0] * n)]
+    lib().call("dn4gl_gather_segments", int(idx.numel()), ptr(idx), ptr(ptr_in), int(ptr_in.numel()) - 1, ptr(ptr_out),
+               ptr(rebase_in), ptr(rebase_out), n, _ptr_array(cols_in), _ptr_array(cols_out),
+               (ctypes.c_int32 * n)(*words), (ctypes.c_int32 * n)(*reb), _stream())

@@ -10,6 +10,8 @@ reference's offline ``tu_data_processing.py`` + ``PYGDataset`` + ``main.py:train
 ``CountingPipeline.step(pattern, graph, counts)`` does the same for the subgraph-counting side
 (train.py:1322-1334 augmentation + train_epoch body :753-838).
 """
+import contextlib
+
 import numpy as np
 import torch
 import torch.nn.functional as F
@@ -251,6 +253,17 @@ class _Pipeline:
         for t in tensors:       # the caching allocator must not recycle them before the train stream is done
             t.record_stream(main)
 
+    @contextlib.contextmanager
+    def _global_batch(self, n):
+        """``global_batch`` = n (when given) for the steps queued inside the block."""
+        prev = self.global_batch
+        if n is not None:
+            self.global_batch = int(n)
+        try:
+            yield
+        finally:
+            self.global_batch = prev
+
     def _step_overlapped(self, transform, train, assume_ready):
         """``train(transform())`` with the transform on the second stream (see ClassificationPipeline.step_resident);
         ``_transform_outputs`` names the tensors of its result that the train stream takes over."""
@@ -410,6 +423,25 @@ class ClassificationPipeline(_Pipeline):
     def step(self, host_batch):
         """host buffers in, python float out: H2D + transform + train step + D2H of the loss (blocking)."""
         return self.step_async(host_batch).result()
+
+    def step_indices(self, ds, idx, global_batch=None):
+        """one train step on graphs `idx` (host integer array) of a ``datasets.ResidentTUDataset``, assembled on the device
+        by ``ds.batch(idx)``; returns a ``PendingLoss`` as ``step_async`` does.  With ``overlap`` the staging copy and the
+        gathers run inside the transform on the second stream, next to the previous train step (the resident columns
+        never change, so nothing waits for the train stream).  In 'conj' mode the batch carries its size hint: with
+        ``num_node_labels`` and ``node_label_min`` given and every graph holding a node, the closed-form CONJ_ builder runs
+        and the step reads nothing back from the device.  global_batch: graphs of the whole data-parallel step (as
+        ``EpochSampler`` yields it); default: this batch times the world size."""
+        def assemble():
+            b = ds.batch(idx)
+            if self.mode != "conj":
+                b.pop("conj_sizes")     # the hint describes the dummy-augmented edge-to-vertex transform only
+            return self.transform(b)
+
+        with self._global_batch(global_batch):
+            if not self.overlap:
+                return PendingLoss(self.train_on(assemble()))
+            return PendingLoss(self._step_overlapped(assemble, self.train_on, assume_ready=True))
 
 
 def _graph_tensors(g):
@@ -613,3 +645,25 @@ class CountingPipeline(_Pipeline):
         p_dev, g_dev = upload(p_host, self.device), upload(g_host, self.device)
         counts = counts_host.to(self.device, non_blocking=True)
         return PendingLoss(self.step_resident(p_dev, g_dev, counts)).result()    # also raises on a builder-kernel error
+
+    def step_indices(self, ds, idx, global_batch=None):
+        """one train step on samples `idx` (host integer array) of a ``datasets.ResidentCountingDataset``, assembled on the
+        device by ``ds.batch(idx)``; returns a ``PendingLoss``.  With ``overlap`` the staging copy and the gathers run with
+        the augmentation on the second stream, next to the previous train step.  The augmentation's own device->host
+        reads (``BatchedGraph.from_batch``) stay.  global_batch: as in ClassificationPipeline.step_indices."""
+        counts = []
+
+        def assemble():
+            p_dev, g_dev, c = ds.batch(idx)
+            counts.append(c)
+            return self.transform(p_dev, g_dev)
+
+        def train(graphs):
+            if self.overlap:        # allocated on the transform stream, read by the train stream
+                counts[0].record_stream(torch.cuda.current_stream())
+            return self.train_on(*graphs, counts[0])
+
+        with self._global_batch(global_batch):
+            if not self.overlap:
+                return PendingLoss(train(assemble()))
+            return PendingLoss(self._step_overlapped(assemble, train, assume_ready=True))

@@ -206,3 +206,39 @@ def random_subisomorphisms(pattern_b, graph_b, seed=0, max_rows=5):
                     m[s, pv] = int(graph_b["dst"][k]) - gn0
         mats.append(m)
     return mats
+
+
+def _unpack(b):
+    """packed batch -> per-graph dicts of the shape ``subgraph_isomorphism.io.read_gml_graph`` returns (graph-local ids)."""
+    out = []
+    for i in range(int(b["num_graphs"])):
+        n0, n1, e0, e1 = (int(b["node_ptr"][i]), int(b["node_ptr"][i + 1]), int(b["edge_ptr"][i]), int(b["edge_ptr"][i + 1]))
+        out.append(dict(num_nodes=n1 - n0, src=b["src"][e0:e1].astype(np.int64) - n0, dst=b["dst"][e0:e1].astype(np.int64) - n0,
+                        vid=b["vid"][n0:n1].astype(np.int64), vlabel=b["vlabel"][n0:n1].astype(np.int64),
+                        elabel=b["elabel"][e0:e1].astype(np.int64), ekey=np.zeros(e1 - e0, np.int64)))
+    return out
+
+
+def counting_samples(shape="small", num_samples=512, seed=0, num_patterns=None):
+    """a counting data set split as ``subgraph_isomorphism.io.load_data`` returns one: a list of ``{id, pattern, graph,
+    subisomorphisms, counts}`` dicts.  num_patterns=None: every sample has its own pattern and graph; otherwise
+    num_patterns patterns share ceil(num_samples / num_patterns) graphs (one sample per pair, the same graph object in
+    every pair that uses it, as in the shared-graph data sets).  Subisomorphisms as ``random_subisomorphisms``."""
+    rng = np.random.default_rng(seed)
+    if num_patterns is None:
+        p, g, counts = counting_batch(shape, num_samples, seed=seed)
+        pats, gras = _unpack(p), _unpack(g)
+        mats = random_subisomorphisms(p, g, seed=seed)
+        return [dict(id="P_%d-G_%d" % (i, i), pattern=pats[i], graph=gras[i], subisomorphisms=mats[i], counts=int(counts[i]))
+                for i in range(num_samples)]
+    n_g = -(-num_samples // num_patterns)
+    p, g, _ = counting_batch(shape, max(num_patterns, n_g), seed=seed)
+    pats, gras = _unpack(p)[:num_patterns], _unpack(g)[:n_g]
+    out = []
+    for k in range(num_samples):
+        pi, gi = k % num_patterns, k // num_patterns
+        S = int(rng.integers(0, 6))
+        m = rng.integers(0, max(gras[gi]["num_nodes"], 1), (S, pats[pi]["num_nodes"]))
+        out.append(dict(id="P_%d-G_%d" % (pi, gi), pattern=pats[pi], graph=gras[gi], subisomorphisms=m,
+                        counts=int(rng.poisson(5.0))))
+    return out

@@ -540,6 +540,22 @@ size_t dn4gl_dot_workspace_bytes(int64_t n);
 int dn4gl_dot_f32(const float *a, const float *b, int64_t n, float *out, void *ws, size_t ws_bytes, int32_t *counter,
                   void *stream);
 
+/* ---- mini-batch assembly from a data set resident in HBM (datasets.py; replaces the host-side collation of PyG's
+ * DataLoader and of GraphAdjDataset.batchify, subgraph_isomorphism/dataset.py:1604-1636) ----------------------------
+ * Segmented gather of one level (nodes, edges, graphs, subisomorphism values) for all of its columns in one launch.
+ * ptr_in[n_seg_in + 1]: the data set's item offsets of the level; idx[K]: the segments to take, each in [0, n_seg_in)
+ * (the caller validates them: an index outside is never read and leaves its output items unwritten); ptr_out[K + 1]:
+ * the batch's offsets (ptr_out[k+1] - ptr_out[k] = ptr_in[idx[k]+1] - ptr_in[idx[k]]).  col_in / col_out: HOST arrays of
+ * ncols (1..8) device column pointers, col_words[c] (host) 4-byte words per item (1 for an int32 / float column, F for
+ * an F-wide float attribute, 2 for int64).  For k < K and j below the segment's length, item ptr_out[k] + j of every
+ * output column is item ptr_in[idx[k]] + j of its input column; in columns with col_rebase[c] != 0 (host) each int32
+ * word also gets rebase_out[k] - rebase_in[idx[k]] added (device arrays; the node offsets on the edge level, so that
+ * src / dst become batch-global node ids).  No allocation, no atomics, deterministic; K == 0 is a no-op.            */
+int dn4gl_gather_segments(int32_t K, const int32_t *idx, const int32_t *ptr_in, int64_t n_seg_in,
+                          const int32_t *ptr_out, const int32_t *rebase_in, const int32_t *rebase_out,
+                          int32_t ncols, const void *const *col_in, void *const *col_out,
+                          const int32_t *col_words, const int32_t *col_rebase, void *stream);
+
 /* ---- small fused elementwise helpers of the layers ------------------------------------------ */
 /* gather rows: out[i,:] = x[idx[i],:] (idx int32, n rows)                                       */
 int dn4gl_gather_rows_f32(const int32_t *idx, const float *x, float *out, int64_t n, int32_t D, void *stream);

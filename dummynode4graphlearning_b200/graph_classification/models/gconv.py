@@ -160,7 +160,9 @@ class GIN(torch.nn.Module):
                 x = ops.apply_gin_mlp(self.first_h, x)
                 out += F.dropout(self.pooling(self.linears[layer](x), data.batch, node_ptr=s.node_ptr), p=self.dropout)
             else:
-                x = self.convs[layer - 1](x, data.edge_index, structure=s)
+                # GINConv reads edge_index only without a compiled structure; a batch from the closed-form CONJ_ builder
+                # would materialise it with a device->host read of the edge count
+                x = self.convs[layer - 1](x, None, structure=s)
                 out += F.dropout(self.linears[layer](self.pooling(x, data.batch, node_ptr=s.node_ptr)),
                                  p=self.dropout, training=self.training)
         return F.log_softmax(out, dim=-1)

@@ -9,7 +9,7 @@ import os
 import torch
 
 from ._lib import lib, ptr
-from .graph import CSR, _stream, require_cuda
+from .graph import CSR, _stream, bind_device, require_cuda
 
 
 def _f32c(t):
@@ -941,3 +941,110 @@ def gather_segments(idx, ptr_in, ptr_out, cols_in, cols_out, rebase=None, rebase
     lib().call("dn4gl_gather_segments", int(idx.numel()), ptr(idx), ptr(ptr_in), int(ptr_in.numel()) - 1, ptr(ptr_out),
                ptr(rebase_in), ptr(rebase_out), n, _ptr_array(cols_in), _ptr_array(cols_out),
                (ctypes.c_int32 * n)(*words), (ctypes.c_int32 * n)(*reb), _stream())
+
+
+# ---- evaluation records and their fixed-order reduction (csrc/eval.cu) ------------------------------------------------
+EVAL_REDUCE_MAX_COLUMNS = 8
+
+
+def _eval_tensor(what, t, dtype, ndim, device=None):
+    """host-side check of one argument of the evaluation kernels (ValueError before any launch)."""
+    if not isinstance(t, torch.Tensor):
+        raise ValueError("%s must be a tensor" % what)
+    if t.dtype != dtype:
+        raise ValueError("%s must be %s, got %s" % (what, dtype, t.dtype))
+    if t.dim() != ndim or not t.is_contiguous():
+        raise ValueError("%s must be a contiguous %d-D tensor, got shape %s" % (what, ndim, tuple(t.shape)))
+    if not t.is_cuda:
+        raise ValueError("%s must live on a CUDA device (there is no CPU path)" % what)
+    if device is not None and t.device != device:
+        raise ValueError("%s is on %s, expected %s" % (what, t.device, device))
+
+
+def _eval_span(what, B, pos0, n):
+    """-> pos0 as an int, checked: the batch's records pos0 .. pos0 + B - 1 lie inside the n-row outputs."""
+    import operator
+    try:
+        pos0 = operator.index(pos0)
+    except TypeError:
+        raise ValueError("%s: pos0 must be an integer, got %r" % (what, pos0)) from None
+    if not (0 <= pos0 and pos0 + B <= n):
+        raise ValueError("%s: records %d .. %d do not fit the %d-row outputs" % (what, pos0, pos0 + B - 1, n))
+    if B > 2 ** 31 - 1:
+        raise ValueError("%s: more than 2^31 - 1 rows in one batch" % what)
+    return pos0
+
+
+def eval_class_rows(logp, y, pos0, pred, nll, correct):
+    """per-graph records of a classification batch (dn4gl_eval_class_rows_f32, one launch): for row b of the (B, C)
+    log-probabilities ``logp`` and the int64 targets ``y``, position ``pos0 + b`` of the split-sized outputs gets
+    ``pred`` (int32 arg-max, lowest index on ties, as ``out.max(1)[1]``), ``nll`` (-logp[b, y[b]]) and ``correct``
+    (1.0 / 0.0).  A target outside [0, C) gives nll 0 and is never correct; a row holding a NaN gives nll NaN and is
+    never correct."""
+    _eval_tensor("eval_class_rows: logp", logp, torch.float32, 2)
+    dev = logp.device
+    B, C = logp.shape
+    if C < 1:
+        raise ValueError("eval_class_rows: logp needs at least one class column")
+    _eval_tensor("eval_class_rows: y", y, torch.int64, 1, dev)
+    if y.numel() != B:
+        raise ValueError("eval_class_rows: %d targets for %d rows" % (y.numel(), B))
+    _eval_tensor("eval_class_rows: pred", pred, torch.int32, 1, dev)
+    _eval_tensor("eval_class_rows: nll", nll, torch.float32, 1, dev)
+    _eval_tensor("eval_class_rows: correct", correct, torch.float32, 1, dev)
+    n = pred.numel()
+    if nll.numel() != n or correct.numel() != n:
+        raise ValueError("eval_class_rows: pred, nll and correct must have the same length")
+    pos0 = _eval_span("eval_class_rows", B, pos0, n)
+    if B == 0:
+        return
+    bind_device(dev)
+    lib().call("dn4gl_eval_class_rows_f32", ptr(logp), ptr(y), B, C, pos0, ptr(pred), ptr(nll), ptr(correct), _stream())
+
+
+def eval_count_rows(pred_c, counts, pos0, pred, err):
+    """per-sample records of a counting batch (dn4gl_eval_count_rows_f32, one launch): for sample b with prediction
+    ``pred_c`` (B or B x 1, float32) and int64 ``counts``, position ``pos0 + b`` of the split-sized outputs gets ``pred``
+    (pred_c itself) and the row ``err`` (n x 3) = |r - t|, (r - t)^2, smooth-L1(r - t) with r = relu(pred_c),
+    t = float(count): the per-element terms of the MAE, MSE and SMSE criteria (losses.eval_criterion)."""
+    if isinstance(pred_c, torch.Tensor) and pred_c.dim() == 2 and pred_c.size(1) == 1:
+        pred_c = pred_c.view(-1)
+    _eval_tensor("eval_count_rows: pred_c", pred_c, torch.float32, 1)
+    dev = pred_c.device
+    B = pred_c.numel()
+    _eval_tensor("eval_count_rows: counts", counts, torch.int64, 1, dev)
+    if counts.numel() != B:
+        raise ValueError("eval_count_rows: %d counts for %d predictions" % (counts.numel(), B))
+    _eval_tensor("eval_count_rows: pred", pred, torch.float32, 1, dev)
+    _eval_tensor("eval_count_rows: err", err, torch.float32, 2, dev)
+    n = pred.numel()
+    if tuple(err.shape) != (n, 3):
+        raise ValueError("eval_count_rows: err must be (%d, 3), got %s" % (n, tuple(err.shape)))
+    pos0 = _eval_span("eval_count_rows", B, pos0, n)
+    if B == 0:
+        return
+    bind_device(dev)
+    lib().call("dn4gl_eval_count_rows_f32", ptr(pred_c), ptr(counts), B, pos0, ptr(pred), ptr(err), _stream())
+
+
+def eval_reduce(v, out=None):
+    """float64 sums of the columns of ``v`` (n, or n x k with 1 <= k <= 8, float32) in an order fixed by n alone
+    (dn4gl_eval_reduce_f32, one launch; n == 0: zeros).  out: a float64 tensor of k elements to write (default: new)."""
+    if isinstance(v, torch.Tensor) and v.dim() == 1:
+        v = v.view(-1, 1)
+    _eval_tensor("eval_reduce: v", v, torch.float32, 2)
+    dev = v.device
+    n, k = v.shape
+    if not 1 <= k <= EVAL_REDUCE_MAX_COLUMNS:
+        raise ValueError("eval_reduce: 1..%d columns, got %d" % (EVAL_REDUCE_MAX_COLUMNS, k))
+    if out is None:
+        out = torch.empty(k, dtype=torch.float64, device=dev)
+    _eval_tensor("eval_reduce: out", out, torch.float64, 1, dev)
+    if out.numel() != k:
+        raise ValueError("eval_reduce: out must hold %d values" % k)
+    bind_device(dev)
+    L = lib()
+    wsb = L.size("dn4gl_eval_reduce_workspace_bytes", n, k)
+    ws, counter = _tc_ws(dev, wsb)
+    L.call("dn4gl_eval_reduce_f32", ptr(v) if n else None, n, k, ptr(out), ptr(ws), wsb, ptr(counter), _stream())
+    return out

@@ -119,6 +119,27 @@ class PendingLoss:
         return self.value
 
 
+class EvalResult:
+    """what ``evaluate`` returns before the device has finished: ``predictions`` (device tensors in the order of the
+    evaluated indices) and the queued float64 sums behind ``metrics()``."""
+
+    def __init__(self, sums, n, finish, predictions):
+        self._sums, self.n, self._finish, self.predictions = sums, n, finish, predictions
+        self._metrics = None
+
+    def metrics(self):
+        """host dict of the split's metrics.  The one device->host read of the evaluation: the column sums together with
+        the builder kernels' sticky error flag, which raises here (as in ``PendingLoss.result()``) instead of returning
+        numbers computed from a malformed batch structure."""
+        if self._metrics is None:
+            host = self._sums.cpu().tolist()
+            if host[-1] != 0:
+                from .graph import check_errors
+                check_errors()          # reads, clears and raises with the code table
+            self._metrics = self._finish(host[:-1], self.n)
+        return dict(self._metrics)
+
+
 class _CapturedGraph:
     """one CUDA graph of ``fn()``, captured on `stream` (default: torch's own capture stream).  ``replay()`` does the
     captured work again and returns what ``fn()`` returned during the capture (static tensors)."""
@@ -278,6 +299,54 @@ class _Pipeline:
         loss = train(out)
         self._mark_step()
         return loss
+
+    def _evaluate(self, ds, idx, batch_size, words, assemble, score, columns, finish):
+        """the shared body of ``evaluate``: validates, then for each batch of the fixed order ``score(assemble(sel),
+        pos0)`` with the model in eval mode under no_grad (assembly on the second stream with ``overlap``).  ``words``:
+        int32 words of the zero-filled record buffer that ``columns(buf)`` cuts into (float32 sum columns, predictions);
+        -> EvalResult."""
+        import torch.distributed as dist
+
+        from .datasets import EpochSampler, _check_indices
+        from .graph import error_flag
+        idx = np.arange(len(ds), dtype=np.int64) if idx is None else _check_indices(idx, len(ds), "evaluate")
+        if idx.size == 0:
+            raise ValueError("evaluate: no samples to evaluate")
+        world, rank = (dist.get_world_size(), dist.get_rank()) if is_distributed() else (1, 0)
+        # the evaluation order is idx itself; each rank takes its contiguous slice of every batch, as in training
+        order = EpochSampler(idx.size, batch_size, shuffle=False, rank=rank, world_size=world)
+        n = int(idx.size)
+        buf = torch.zeros(words(n), dtype=torch.int32, device=self.device)
+        sum_cols, predictions = columns(buf, n)
+        modes = [(m, m.training) for m in self.model.modules()]
+        self.model.eval()
+        try:
+            with torch.no_grad():
+                for pos, _ in order.batches():
+                    if len(pos) == 0:           # a short last batch leaves this rank nothing
+                        self._eval_skip()
+                        continue
+                    sel, pos0 = idx[pos], int(pos[0])
+                    if not self.overlap:
+                        score(assemble(sel), pos0)
+                    else:
+                        self._step_overlapped(lambda: assemble(sel), lambda out: score(out, pos0), assume_ready=True)
+        finally:
+            for m, training in modes:
+                m.training = training
+        if world > 1:
+            # every rank wrote its own positions only; as int32 words the sum adds exact zeros to every bit pattern
+            # (NaN included), so all ranks hold the same records, bit for bit
+            dist.all_reduce(buf)
+        k = [1 if c.dim() == 1 else c.size(1) for c in sum_cols]
+        sums = torch.empty(sum(k) + 1, dtype=torch.float64, device=self.device)
+        for col, o in zip(sum_cols, np.cumsum([0] + k[:-1])):
+            ops.eval_reduce(col, sums[int(o):int(o) + col.numel() // n])
+        sums[-1:].copy_(error_flag(self.device))
+        return EvalResult(sums, n, finish, predictions)
+
+    def _eval_skip(self):
+        """a batch of the evaluation order that holds nothing for this rank (collectives the others issue go here)."""
 
 
 class ClassificationPipeline(_Pipeline):
@@ -442,6 +511,55 @@ class ClassificationPipeline(_Pipeline):
             if not self.overlap:
                 return PendingLoss(self.train_on(assemble()))
             return PendingLoss(self._step_overlapped(assemble, self.train_on, assume_ready=True))
+
+    def evaluate(self, ds, idx=None, batch_size=512, log_probs=False):
+        """accuracy and mean NLL of the model over graphs `idx` (host integer array; default: every graph, in order) of a
+        ``datasets.ResidentTUDataset`` -- the reference's ``eval_test`` (main.py:54, 90-104), whose numbers drive early
+        stopping and the choice of ``best.pt``.  Returns an ``EvalResult`` as soon as the work is queued:
+        ``metrics()`` -> ``{"accuracy", "loss"}`` (correct / n and the summed ``F.nll_loss`` / n); ``predictions`` ->
+        ``pred`` (int32 arg-max, ``out.max(1)[1]``), ``nll`` (per graph) and, with ``log_probs``, the (n, C)
+        log-probabilities, all in the order of `idx`.
+
+        Batches of ``batch_size`` graphs in the order of `idx` are assembled by ``ds.batch``, transformed, and scored by
+        the model's own eval-mode forward under ``torch.no_grad()``; one kernel writes each batch's records at its offset
+        and one fixed-order reduction per column gives the sums, so the metrics do not depend on the batching.  The
+        model's train / eval modes are restored afterwards; no parameter, BatchNorm buffer or optimizer state changes.
+        Under torch.distributed each rank scores its contiguous slice of every batch and the records are all-reduced:
+        every rank returns the same bits.  Kept from the reference: GIN's layer-0 dropout is applied without
+        ``training=`` (gconv.py:210), so with ``dropout_ratio > 0`` the scores are random, as there."""
+        C = getattr(self.model, "num_classes", None)
+        if log_probs and not C:
+            raise ValueError("evaluate(log_probs=True) needs a model with num_classes")
+        rec = {}
+
+        def columns(buf, n):
+            rec["pred"] = buf[:n]
+            rec["nll"], rec["correct"] = buf[n:2 * n].view(torch.float32), buf[2 * n:3 * n].view(torch.float32)
+            preds = dict(pred=rec["pred"], nll=rec["nll"])
+            if log_probs:
+                preds["log_probs"] = rec["log_probs"] = buf[3 * n:].view(torch.float32).view(n, C)
+            return [rec["correct"], rec["nll"]], preds
+
+        def assemble(sel):
+            b = ds.batch(sel)
+            if self.mode != "conj":
+                b.pop("conj_sizes")
+            # the eager transform, also where train steps replay a captured one: a captured transform writes static
+            # buffers that the next train step reads (the _consumed protocol), and evaluation batches would take
+            # signatures in the train-time cache; the eager transform shares nothing with training
+            return self._transform_eager(b)
+
+        def score(data, pos0):
+            out = self.model(data)
+            ops.eval_class_rows(out, data.y.long(), pos0, rec["pred"], rec["nll"], rec["correct"])
+            if log_probs:
+                rec["log_probs"][pos0:pos0 + out.size(0)].copy_(out)
+
+        def finish(s, n):
+            return {"accuracy": s[0] / n, "loss": s[1] / n}
+
+        return self._evaluate(ds, idx, batch_size, lambda n: (3 + (C if log_probs else 0)) * n, assemble, score,
+                              columns, finish)
 
 
 def _graph_tensors(g):
@@ -667,3 +785,42 @@ class CountingPipeline(_Pipeline):
             if not self.overlap:
                 return PendingLoss(train(assemble()))
             return PendingLoss(self._step_overlapped(assemble, train, assume_ready=True))
+
+    def evaluate(self, ds, idx=None, batch_size=512):
+        """the reference's ``evaluate`` (train.py:609-618 criteria) over samples `idx` (host integer array; default: every
+        sample, in order) of a ``datasets.ResidentCountingDataset``; returns an ``EvalResult`` as soon as the work is
+        queued: ``metrics()`` -> ``{"MAE", "MSE", "SMSE", "RMSE"}`` (``losses.eval_criterion`` over the whole split:
+        relu(pred_c) against the counts; RMSE = sqrt(MSE)); ``predictions`` -> ``pred_c`` in the order of `idx`.
+
+        Batching, records, reduction, modes and distributed behaviour as in ``ClassificationPipeline.evaluate``; the
+        augmentation's own device->host reads (``BatchedGraph.from_batch``) stay.  Kept from the reference: the
+        prediction head's L * bias term depends on the batch's padded length (SURVEY.md App. A-7), so a sample's
+        prediction depends on which samples share its batch; under torch.distributed ``exact_sharding`` pads every
+        rank's slice to the whole batch's lengths, as in training."""
+        rec, counts = {}, []
+
+        def columns(buf, n):
+            rec["pred"] = buf[:n].view(torch.float32)
+            rec["err"] = buf[n:].view(torch.float32).view(n, 3)
+            return [rec["err"]], dict(pred_c=rec["pred"])
+
+        def assemble(sel):
+            p_dev, g_dev, c = ds.batch(sel)
+            counts.append(c)
+            return self.transform(p_dev, g_dev)
+
+        def score(graphs, pos0):
+            c = counts.pop()
+            if self.overlap:        # allocated on the transform stream, read here
+                c.record_stream(torch.cuda.current_stream())
+            out = self.model(*graphs)
+            ops.eval_count_rows(out["pred_c"], c, pos0, rec["pred"], rec["err"])
+
+        def finish(s, n):
+            return {"MAE": s[0] / n, "MSE": s[1] / n, "SMSE": s[2] / n, "RMSE": float(np.sqrt(s[1] / n))}
+
+        return self._evaluate(ds, idx, batch_size, lambda n: 4 * n, assemble, score, columns, finish)
+
+    def _eval_skip(self):
+        if self.exact_sharding and is_distributed():    # the other ranks agree on this batch's padded lengths
+            sync_padded_lengths(0, 0, 0, 0)

@@ -556,6 +556,28 @@ int dn4gl_gather_segments(int32_t K, const int32_t *idx, const int32_t *ptr_in, 
                           int32_t ncols, const void *const *col_in, void *const *col_out,
                           const int32_t *col_words, const int32_t *col_rebase, void *stream);
 
+/* ---- evaluation over a held-out split (pipelines.py evaluate; the reference's eval_test, main.py:54, and evaluate,
+ * subgraph_isomorphism/train.py:609-618) ----------------------------------------------------------------------------
+ * Record kernels write one record per sample of a batch at positions pos0 .. pos0 + B - 1 of split-sized arrays.
+ * dn4gl_eval_class_rows_f32: logp (B, C) row-major log-probabilities, y[B] int64 targets.  pred[p] = arg-max of the
+ *   row as torch.max(dim=1) picks it (lowest index on ties; a NaN counts as the largest value, the first NaN wins);
+ *   nll[p] = -logp[b, y[b]]; correct[p] = 1.f if pred == y else 0.f.  A y outside [0, C) contributes nll 0 and is never
+ *   correct (as in dn4gl_nll_mean_f32).  A row holding a NaN gets nll = NaN and correct = 0, whatever its target.
+ * dn4gl_eval_count_rows_f32: pred_c[B] fp32, counts[B] int64; with r = relu(pred_c), t = (float)count:
+ *   pred[p] = pred_c[b]; err[3p .. 3p+2] = { |r - t|, (r - t)^2, smooth-L1(r - t, beta 1) } (F.l1_loss / F.mse_loss /
+ *   F.smooth_l1_loss per element).
+ * dn4gl_eval_reduce_f32: out[c] = sum_{i < n} v[i * k + c] in double for k (1..8) interleaved fp32 columns.  The order
+ *   is fixed by n alone (tiles of 1024 rows summed by a fixed tree, tile partials merged in tile order by a fixed tree;
+ *   csrc/eval.cu), not by the grid or the SM count.  ws: dn4gl_eval_reduce_workspace_bytes(n, k) bytes, 8-byte
+ *   aligned; counter: one int32 that is 0 on entry (left 0).  n == 0 writes k zeros and reads nothing.              */
+int dn4gl_eval_class_rows_f32(const float *logp, const int64_t *y, int32_t B, int32_t C, int64_t pos0, int32_t *pred,
+                              float *nll, float *correct, void *stream);
+int dn4gl_eval_count_rows_f32(const float *pred_c, const int64_t *counts, int32_t B, int64_t pos0, float *pred,
+                              float *err, void *stream);
+size_t dn4gl_eval_reduce_workspace_bytes(int64_t n, int32_t k);
+int dn4gl_eval_reduce_f32(const float *v, int64_t n, int32_t k, double *out, void *ws, size_t ws_bytes,
+                          int32_t *counter, void *stream);
+
 /* ---- small fused elementwise helpers of the layers ------------------------------------------ */
 /* gather rows: out[i,:] = x[idx[i],:] (idx int32, n rows)                                       */
 int dn4gl_gather_rows_f32(const int32_t *idx, const float *x, float *out, int64_t n, int32_t D, void *stream);

@@ -289,13 +289,14 @@ class ResidentCountingDataset:
             m = np.asarray(x["subisomorphisms"], dtype=np.int64)
             mats.append(m.reshape(-1, x["pattern"]["num_nodes"]) if m.ndim != 2 else m)
         self._val_sizes = np.asarray([m.size for m in mats], np.int64)
+        self._rows = np.asarray([m.shape[0] for m in mats], np.int64)    # host copy: the dummy column's offsets
         val_ptr = _offsets(self._val_sizes)
         if val_ptr[-1] > _I32_MAX:
             raise ValueError("ResidentCountingDataset: more than 2^31 - 1 subisomorphism entries")
         values = np.concatenate([m.reshape(-1) for m in mats]) if mats else np.zeros(0, np.int64)
-        cols = T.to_device(dict(val_ptr=val_ptr, values=values, rows=np.asarray([m.shape[0] for m in mats], np.int64),
+        cols = T.to_device(dict(val_ptr=val_ptr, values=values, rows=self._rows,
                                 sample_ptr=np.arange(self.num_samples + 1)), self.device)
-        self._val_ptr, self._sample_ptr, self._values, self._rows = (cols[k] for k in ("val_ptr", "sample_ptr", "values", "rows"))
+        self._val_ptr, self._sample_ptr, self._values, self._rows_d = (cols[k] for k in ("val_ptr", "sample_ptr", "values", "rows"))
         self._counts = torch.as_tensor(np.asarray([int(x["counts"]) for x in samples], np.int64)).to(self.device)
         self._staging = _Staging()
         torch.cuda.synchronize(self.device)
@@ -303,9 +304,11 @@ class ResidentCountingDataset:
     def __len__(self):
         return self.num_samples
 
-    def batch(self, idx, subisomorphisms=False):
+    def batch(self, idx, subisomorphisms=False, dummy_column=False):
         """device batch of samples `idx` (host integer array, validated here: ValueError before any device work); queued
-        on the current stream: one host->device copy and 5 gather launches (6 with subisomorphisms)."""
+        on the current stream: one host->device copy and 5 gather launches (6 with subisomorphisms).  dummy_column (with
+        subisomorphisms): the subisomorphisms come with the dummy column ``add_dummy_nodes_edges`` appends
+        (``matching.append_dummy_column``, one more launch; its offsets are computed here on the host)."""
         idx = _check_indices(idx, self.num_samples, "ResidentCountingDataset")
         K = len(idx)
         P, G = self._pid[idx], self._gid[idx]
@@ -314,17 +317,24 @@ class ResidentCountingDataset:
         parts = [idx, P, G, pn, pe, gn, ge, np.arange(K + 1)]
         if subisomorphisms:
             val_ptr = _offsets(self._val_sizes[idx])
-            if val_ptr[-1] > _I32_MAX:
-                raise ValueError("ResidentCountingDataset: the batch exceeds 2^31 - 1 subisomorphism entries")
             parts.append(val_ptr)
+            if dummy_column:
+                from .subgraph_isomorphism.matching import dummy_column_offsets
+                parts.append(dummy_column_offsets(self._val_sizes[idx], self._rows[idx]))
+            if parts[-1][-1] > _I32_MAX:
+                raise ValueError("ResidentCountingDataset: the batch exceeds 2^31 - 1 subisomorphism entries")
         views = self._staging.upload(parts, self.device)
         idx_d, P_d, G_d, pn_d, pe_d, gn_d, ge_d, sp_d = views[:8]
         p_dev = self.patterns.gather(P_d, pn_d, pe_d, pn[-1], pe[-1])
         g_dev = self.graphs.gather(G_d, gn_d, ge_d, gn[-1], ge[-1])
-        per_sample = dict(counts=self._counts, rows=self._rows) if subisomorphisms else dict(counts=self._counts)
+        per_sample = dict(counts=self._counts, rows=self._rows_d) if subisomorphisms else dict(counts=self._counts)
         s = _gather_level(idx_d, self._sample_ptr, sp_d, per_sample, K)
         if not subisomorphisms:
             return p_dev, g_dev, s["counts"]
         vp_d = views[8]
         v = _gather_level(idx_d, self._val_ptr, vp_d, dict(values=self._values), val_ptr[-1])
-        return p_dev, g_dev, s["counts"], dict(val_ptr=vp_d, values=v["values"], rows=s["rows"])
+        sub = dict(val_ptr=vp_d, values=v["values"], rows=s["rows"])
+        if dummy_column:
+            from .subgraph_isomorphism.matching import append_dummy_column
+            sub = append_dummy_column(sub, g_dev, views[9], int(parts[-1][-1]))
+        return p_dev, g_dev, s["counts"], sub

@@ -1048,3 +1048,123 @@ def eval_reduce(v, out=None):
     ws, counter = _tc_ws(dev, wsb)
     L.call("dn4gl_eval_reduce_f32", ptr(v) if n else None, n, k, ptr(out), ptr(ws), wsb, ptr(counter), _stream())
     return out
+
+
+# ---- the matching objective of the counting models (csrc/match.cu) -----------------------------------------------------
+MATCH_CRITERIA = {"MAE": 0, "MSE": 1, "SMSE": 2}       # losses._CRITERIA: F.l1_loss, F.mse_loss, F.smooth_l1_loss
+
+
+def _i32_vector(what, t, n=None, device=None):
+    _eval_tensor(what, t, torch.int32, 1, device)
+    if n is not None and t.numel() != n:
+        raise ValueError("%s must hold %d values, got %d" % (what, n, t.numel()))
+
+
+def subiso_append_dummy(val_ptr, values, rows, g_node_ptr, out_ptr, out_total):
+    """the dummy column of a packed subisomorphism batch (dn4gl_subiso_append_dummy, one launch): row s of sample b
+    becomes its np_b ids followed by n_b = g_node_ptr[b + 1] - g_node_ptr[b] (the graph's node count BEFORE
+    augmentation), written at ``out_ptr[b] + s * (np_b + 1)``.  All arguments int32 device tensors; out_ptr (B + 1) holds
+    the output offsets ``val_ptr[b] + sum_{b' < b} rows[b']`` and out_total = out_ptr[B], both computed by the caller on
+    the host (``matching.dummy_column_offsets``).  -> int32 (out_total,)."""
+    _i32_vector("subiso_append_dummy: val_ptr", val_ptr)
+    dev = val_ptr.device
+    B = val_ptr.numel() - 1
+    if B < 0:
+        raise ValueError("subiso_append_dummy: val_ptr needs B + 1 >= 1 offsets")
+    _i32_vector("subiso_append_dummy: values", values, None, dev)
+    _i32_vector("subiso_append_dummy: rows", rows, B, dev)
+    _i32_vector("subiso_append_dummy: g_node_ptr", g_node_ptr, B + 1, dev)
+    _i32_vector("subiso_append_dummy: out_ptr", out_ptr, B + 1, dev)
+    out_total = int(out_total)
+    if not values.numel() <= out_total <= 2 ** 31 - 1:
+        raise ValueError("subiso_append_dummy: out_total %d is outside [%d, 2^31 - 1]" % (out_total, values.numel()))
+    out = torch.empty(out_total, dtype=torch.int32, device=dev)
+    if B == 0 or out_total == 0:
+        return out
+    bind_device(dev)
+    lib().call("dn4gl_subiso_append_dummy", B, ptr(val_ptr), ptr(values), ptr(rows), ptr(g_node_ptr), ptr(out_ptr),
+               out_total, ptr(out), _stream())
+    return out
+
+
+def _match_kind(what, pred, mask, weights, seg_ptr, B, dev):
+    """checked (pred, mask, weights, seg_ptr, L) of one kind of the match terms, or None when the kind is left out."""
+    if pred is None or weights is None:
+        return None
+    if isinstance(pred, torch.Tensor) and isinstance(mask, torch.Tensor):
+        pred, mask = pred.contiguous(), mask.contiguous()
+    _eval_tensor(what + " prediction", pred, torch.float32, 2, dev)
+    if pred.size(0) != B:
+        raise ValueError("match_loss: %s prediction has %d rows for %d graphs" % (what, pred.size(0), B))
+    L = pred.size(1)
+    _eval_tensor(what + " mask", mask, torch.bool, 2, dev)
+    if tuple(mask.shape) != (B, L):
+        raise ValueError("match_loss: %s mask must be (%d, %d), got %s" % (what, B, L, tuple(mask.shape)))
+    _i32_vector("match_loss: %s seg_ptr" % what, seg_ptr, B + 1, dev)
+    if not isinstance(weights, torch.Tensor) or weights.dtype not in (torch.int32, torch.int64):
+        raise ValueError("match_loss: %s weights must be an int32 or int64 tensor" % what)
+    weights = weights.to(torch.int32) if weights.dtype == torch.int64 else weights
+    _i32_vector("match_loss: %s weights" % what, weights, None, dev)
+    return pred, mask, weights, seg_ptr, L
+
+
+def _kind_args(k):
+    return (None, None, None, None, 0) if k is None else (ptr(k[0]), ptr(k[1]), ptr(k[2]), ptr(k[3]), k[4])
+
+
+class _MatchLoss(torch.autograd.Function):
+    """match_loss_w * (loss_v + loss_e) + match_reg_w * (reg_v + reg_e) as one kernel each way (csrc/match.cu)."""
+
+    @staticmethod
+    def forward(ctx, pred_c, pred_v, pred_e, kv, ke, crit, scalars):
+        dev = pred_c.device
+        B = pred_c.size(0)
+        L = lib()
+        out = torch.empty((), dtype=torch.float32, device=dev)
+        wsb = L.size("dn4gl_match_loss_workspace_bytes", B)
+        ws, counter = _tc_ws(dev, wsb)
+        L.call("dn4gl_match_loss_f32", B, ptr(pred_c), *_kind_args(kv), *_kind_args(ke), crit, *(ptr(s) for s in scalars),
+               ptr(out), ptr(ws), wsb, ptr(counter), _stream())
+        ctx.kv, ctx.ke, ctx.crit, ctx.scalars, ctx.B = kv, ke, crit, scalars, B
+        ctx.shape_c = pred_c.shape
+        ctx.pred_c = pred_c
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        g = _f32c(g).reshape(1)
+        kv, ke = ctx.kv, ctx.ke
+        gc = torch.empty(ctx.shape_c, dtype=torch.float32, device=g.device)
+        gv = None if kv is None else torch.empty_like(kv[0])
+        ge = None if ke is None else torch.empty_like(ke[0])
+        lib().call("dn4gl_match_loss_bwd_f32", ctx.B, ptr(g), ptr(ctx.pred_c), *_kind_args(kv), *_kind_args(ke), ctx.crit,
+                   *(ptr(s) for s in ctx.scalars), ptr(gv), ptr(ge), ptr(gc), _stream())
+        return gc, gv, ge, None, None, None, None
+
+
+def match_loss(pred_c, pred_v, mask_v, node_weights, node_ptr, pred_e, mask_e, edge_weights, edge_ptr, bp_loss, neg_slp,
+               match_loss_w, match_reg_w):
+    """the match terms of the counting models' bp_loss (losses.counting_bp_loss with the identity refine_*_weights) as a
+    0-d float32 tensor with a gradient for pred_c (B, 1), pred_v and pred_e: dn4gl_match_loss_f32 / _bwd_f32, one launch
+    each way.  pred_v / pred_e: the model's left-padded (B, L) predictions with its own g_v_mask / g_e_mask; node_weights /
+    edge_weights: the FLAT int32 (or int64) weights of the augmented graph batch with their row offsets node_ptr /
+    edge_ptr (left-padded on the fly, no (B, L) target is built).  A kind whose prediction or weights are None is left
+    out.  neg_slp, match_loss_w, match_reg_w: float32 device scalars read by the kernels (a captured step follows
+    changes to them)."""
+    if bp_loss not in MATCH_CRITERIA:
+        raise NotImplementedError(bp_loss)
+    if isinstance(pred_c, torch.Tensor):
+        pred_c = pred_c.contiguous()
+    if isinstance(pred_c, torch.Tensor) and pred_c.dim() == 2 and pred_c.size(1) == 1:
+        _eval_tensor("match_loss: pred_c", pred_c, torch.float32, 2)
+    else:
+        _eval_tensor("match_loss: pred_c", pred_c, torch.float32, 1)
+    dev = pred_c.device
+    B = pred_c.size(0)
+    for what, s in (("neg_slp", neg_slp), ("match_loss_w", match_loss_w), ("match_reg_w", match_reg_w)):
+        _eval_tensor("match_loss: " + what, s, torch.float32, 0, dev)
+    kv = _match_kind("node", pred_v, mask_v, node_weights, node_ptr, B, dev)
+    ke = _match_kind("edge", pred_e, mask_e, edge_weights, edge_ptr, B, dev)
+    bind_device(dev)
+    return _MatchLoss.apply(pred_c, None if kv is None else kv[0], None if ke is None else ke[0], kv, ke,
+                            MATCH_CRITERIA[bp_loss], (neg_slp, match_loss_w, match_reg_w))

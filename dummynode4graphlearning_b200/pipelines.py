@@ -582,11 +582,12 @@ def _graph_tensors(g):
     return tensors, scalars
 
 
-def _counting_tensors(pattern, graph, counts):
-    """every device tensor a counting train step reads (fixed order) + the host scalars of its CUDA-graph signature."""
+def _counting_tensors(pattern, graph, counts, node_weights=None, edge_weights=None):
+    """every device tensor a counting train step reads (fixed order) + the host scalars of its CUDA-graph signature.  The
+    match weights are among the tensors (None when absent), so a matched step has a signature of its own."""
     tp, sp = _graph_tensors(pattern)
     tg, sg = _graph_tensors(graph)
-    return tp + tg + [counts], [tuple(sp), tuple(sg)]
+    return tp + tg + [counts, node_weights, edge_weights], [tuple(sp), tuple(sg)]
 
 
 def _static_graph(g):
@@ -604,10 +605,30 @@ def _static_graph(g):
     return c
 
 
+def _match_kinds(match_weights):
+    """the reference's --match_weights flag (None, "node", "edge", "node,edge") -> (node, edge) booleans."""
+    if match_weights is None:
+        return None
+    kinds = [k.strip() for k in str(match_weights).split(",")]
+    if not kinds or any(k not in ("node", "edge") for k in kinds) or len(set(kinds)) != len(kinds):
+        raise ValueError("match_weights: None, 'node', 'edge' or 'node,edge', got %r" % (match_weights,))
+    return "node" in kinds, "edge" in kinds
+
+
+def _check_identity_refine(model):
+    """the fused match loss reads the weights as they are: refuse a model that refines them."""
+    from .subgraph_isomorphism.models.basemodel import _CountingBase
+    for name in ("refine_node_weights", "refine_edge_weights"):
+        if getattr(type(model), name, None) is not getattr(_CountingBase, name):
+            raise ValueError("match weights: %s overrides %s; the fused match loss reads the weights unrefined"
+                             % (type(model).__name__, name))
+
+
 class CountingPipeline(_Pipeline):
     def __init__(self, model, optimizer, config, add_dummy=True, rep_reg_w=0.0, neg_slp=0.01, max_grad_norm=8.0,
                  cuda_graphs=None, max_graphs=8, overlap=None, exact_sharding=False, bp_loss="MSE", match_loss_w=0.0,
-                 match_reg_w=0.0, remove_loops=False, add_rev=False, convert_conj=False, share_emb_net=True):
+                 match_reg_w=0.0, remove_loops=False, add_rev=False, convert_conj=False, share_emb_net=True,
+                 match_weights=None):
         """config: the dataset maxima BEFORE augmentation (max_npv ... max_ngel).  cuda_graphs / overlap: as in
         ClassificationPipeline (defaults: graphs on exactly when the optimizer was built with capturable=True, the
         augmentation + CSR builds on a second stream exactly when graphs are on).  exact_sharding: under
@@ -615,19 +636,34 @@ class CountingPipeline(_Pipeline):
         host read per step) so that a sharded batch gives exactly the single-process head / filter numbers
         (SURVEY.md 8(e) i, v); off by default -- each rank then pads to its own shard's maxima.  bp_loss / match_loss_w /
         match_reg_w: criterion and weights of the match terms (train.py:620-627, 776-813); they only enter steps that
-        are given per-node / per-edge match weights (``train_on(..., node_weights=, edge_weights=)``), which run
-        eagerly (the targets change with every mini-batch).  remove_loops / add_rev / convert_conj: the reference's other
+        are given per-node / per-edge match weights (``train_on(..., node_weights=, edge_weights=)``, or ``step_indices``
+        with ``match_weights``).  Such steps compute the match terms with one kernel each way (``ops.match_loss``) and
+        are captured and replayed like the others: the weights are among the tensors a replay copies in, and
+        match_loss_w / match_reg_w live in device scalars like neg_slp.  match_weights: the reference's --match_weights
+        (None, "node", "edge", "node,edge"): ``step_indices`` then also gathers the samples' subisomorphisms, appends the
+        dummy column (with add_dummy) and trains on the match-weight targets of the augmented batch
+        (``matching.node_weights`` / ``edge_weights``).  Refused with convert_conj, and for a model that overrides
+        ``refine_node_weights`` / ``refine_edge_weights``.  remove_loops / add_rev / convert_conj: the reference's other
         data-set level preprocessing switches, applied per mini-batch on the GPU in the reference's order
         (train.py:1271-1340: loops, reversed edges, dummy, edge-to-vertex), each with the maxima the previous steps
         leave behind; build the model with ``transforms.process_model_config`` of the same switches."""
+        self.match_weights = _match_kinds(match_weights)
+        if self.match_weights is not None:
+            if convert_conj:
+                raise ValueError("match_weights with convert_conj: the conjugate graph's node-weight numbering is not "
+                                 "pinned against the reference")
+            _check_identity_refine(model)
         super().__init__(model, optimizer, cuda_graphs, max_graphs, overlap)
         self.cfg, self.add_dummy = config, add_dummy
         # neg_slp and rep_reg_w change every step in the reference (train.py:648-740 recomputes them from their
         # schedules): they live in device scalars that the (possibly captured) train step READS, so an update through the
         # properties below is seen by the next step / CUDA-graph replay
+        # (match_reg_w too: anneal_cosine$0.01$0.0 by default, losses.py:30)
         self._neg_slp_t = torch.zeros((), dtype=torch.float32, device=self.device)
         self._rep_reg_w_t = torch.zeros((), dtype=torch.float32, device=self.device)
-        self._neg_slp = self._rep_reg_w = None
+        self._match_loss_w_t = torch.zeros((), dtype=torch.float32, device=self.device)
+        self._match_reg_w_t = torch.zeros((), dtype=torch.float32, device=self.device)
+        self._neg_slp = self._rep_reg_w = self._match_loss_w = self._match_reg_w = None
         self.neg_slp, self.rep_reg_w, self.max_grad_norm = neg_slp, rep_reg_w, max_grad_norm
         self.share_emb_net = bool(share_emb_net)
         self.exact_sharding = bool(exact_sharding)
@@ -654,6 +690,26 @@ class CountingPipeline(_Pipeline):
             self._rep_reg_w = float(v)
             self._rep_reg_w_t.fill_(self._rep_reg_w)
 
+    @property
+    def match_loss_w(self):
+        return self._match_loss_w
+
+    @match_loss_w.setter
+    def match_loss_w(self, v):
+        if v != self._match_loss_w:
+            self._match_loss_w = float(v)
+            self._match_loss_w_t.fill_(self._match_loss_w)
+
+    @property
+    def match_reg_w(self):
+        return self._match_reg_w
+
+    @match_reg_w.setter
+    def match_reg_w(self, v):
+        if v != self._match_reg_w:
+            self._match_reg_w = float(v)
+            self._match_reg_w_t.fill_(self._match_reg_w)
+
     def augment(self, p_dev, g_dev):
         """flat device batches -> flat device batches after the configured preprocessing switches (no CSR yet)."""
         c = self.cfg
@@ -674,7 +730,10 @@ class CountingPipeline(_Pipeline):
         return p_dev, g_dev
 
     def transform(self, p_dev, g_dev):
-        p_dev, g_dev = self.augment(p_dev, g_dev)
+        return self._compile(*self.augment(p_dev, g_dev))
+
+    def _compile(self, p_dev, g_dev):
+        """augmented flat batches -> BatchedGraph pair with both CSRs (and the shared padded lengths)."""
         pattern, graph = BatchedGraph.from_batch(p_dev, self.device), BatchedGraph.from_batch(g_dev, self.device)
         for g in (pattern, graph):   # compile both CSRs + degrees now (calculate_degrees, train.py:1355-1356)
             g.in_degrees()
@@ -703,12 +762,27 @@ class CountingPipeline(_Pipeline):
 
     def match_loss_fn(self, out, counts, graph, node_weights, edge_weights):
         """the reference's full bp_loss (losses.counting_bp_loss) with flat per-node / per-edge match weights of the
-        augmented graph batch (matching.node_weights / edge_weights), left-padded here like the model's outputs."""
+        augmented graph batch (matching.node_weights / edge_weights), left-padded here like the model's outputs.  The
+        tensor restatement of what a matched train step computes with ``fused_loss_fn``; it zeroes out["pred_v"] /
+        out["pred_e"] on masked positions in place, as the reference does."""
         from .subgraph_isomorphism.losses import counting_bp_loss, pad_match_weights
         nw = None if node_weights is None else pad_match_weights(node_weights, graph.node_ptr, graph.padded_num_nodes())
         ew = None if edge_weights is None else pad_match_weights(edge_weights, graph.edge_ptr, graph.padded_num_edges())
         return counting_bp_loss(out, counts, nw, ew, model=self.model, bp_loss=self.bp_loss, neg_slp=self.neg_slp,
                                 rep_reg_w=self.rep_reg_w, match_loss_w=self.match_loss_w, match_reg_w=self.match_reg_w)[0]
+
+    def fused_loss_fn(self, out, counts, graph, node_weights, edge_weights):
+        """``match_loss_fn``'s value with the match terms from ``ops.match_loss`` (one kernel each way, flat weights read
+        in place, every weight and the slope from device scalars); the model's outputs are left unchanged.  A kind
+        whose weights or prediction is None contributes nothing (losses.py:95-96)."""
+        loss = self.loss_fn(out, counts)
+        pv = out.get("pred_v") if node_weights is not None else None
+        pe = out.get("pred_e") if edge_weights is not None else None
+        if pv is None and pe is None:
+            return loss
+        return loss + ops.match_loss(out["pred_c"], pv, out.get("g_v_mask"), node_weights, graph.node_ptr, pe,
+                                     out.get("g_e_mask"), edge_weights, graph.edge_ptr, self.bp_loss, self._neg_slp_t,
+                                     self._match_loss_w_t, self._match_reg_w_t)
 
     def _train_body(self, pattern, graph, counts, node_weights=None, edge_weights=None):
         self.bucket.zero()
@@ -716,7 +790,7 @@ class CountingPipeline(_Pipeline):
         if node_weights is None and edge_weights is None:
             loss = self.loss_fn(out, counts)
         else:
-            loss = self.match_loss_fn(out, counts, graph, node_weights, edge_weights)
+            loss = self.fused_loss_fn(out, counts, graph, node_weights, edge_weights)
         loss.backward()
         self.bucket.gather()
         if is_distributed():
@@ -733,23 +807,27 @@ class CountingPipeline(_Pipeline):
         if not self.model.training:      # Module.train() walks every submodule (~0.2 ms of host time per step)
             self.model.train()
         if node_weights is not None or edge_weights is not None:
-            return self._train_body(pattern, graph, counts, node_weights, edge_weights)
+            _check_identity_refine(self.model)
         if not self.cuda_graphs:
-            return self._train_body(pattern, graph, counts)
-        tensors, scalars = _counting_tensors(pattern, graph, counts)
+            return self._train_body(pattern, graph, counts, node_weights, edge_weights)
+        tensors, scalars = _counting_tensors(pattern, graph, counts, node_weights, edge_weights)
         ent = self._captured(self._graphs, _signature(tensors, scalars), lambda: _CapturedStep(
-            self._train_body, (_static_graph(pattern), _static_graph(graph), counts.clone()), _counting_tensors))
+            self._train_body, (_static_graph(pattern), _static_graph(graph), counts.clone(),
+                               *(None if w is None else w.clone() for w in (node_weights, edge_weights))),
+            _counting_tensors))
         if ent is None:
-            return self._train_body(pattern, graph, counts)
+            return self._train_body(pattern, graph, counts, node_weights, edge_weights)
         ent.load(tensors)
         return ent.replay()
 
-    def _transform_outputs(self, graphs):
-        """every device tensor of both graphs; everything the captured step copies out of the batch exists before the
-        hand-over (the CSRs are built here, on the transform's stream, if the transform left one out)."""
+    def _transform_outputs(self, out):
+        """every device tensor of both graphs (out[:2]) and the match weights that may follow them; everything the
+        captured step copies out of the batch exists before the hand-over (the CSRs are built here, on the transform's
+        stream, if the transform left one out)."""
+        graphs = out[:2]
         for g in graphs:
             g.csr_in, g.csr_out
-        return [t for g in graphs for t in _graph_tensors(g)[0] if t is not None]
+        return [t for g in graphs for t in _graph_tensors(g)[0] if t is not None] + [t for t in out[2:] if t is not None]
 
     def step_resident(self, p_dev, g_dev, counts_dev, assume_ready=False):
         """see ClassificationPipeline.step_resident: with ``overlap`` the augmentation + CSR builds of this mini-batch run
@@ -768,18 +846,31 @@ class CountingPipeline(_Pipeline):
         """one train step on samples `idx` (host integer array) of a ``datasets.ResidentCountingDataset``, assembled on the
         device by ``ds.batch(idx)``; returns a ``PendingLoss``.  With ``overlap`` the staging copy and the gathers run with
         the augmentation on the second stream, next to the previous train step.  The augmentation's own device->host
-        reads (``BatchedGraph.from_batch``) stay.  global_batch: as in ClassificationPipeline.step_indices."""
+        reads (``BatchedGraph.from_batch``) stay.  global_batch: as in ClassificationPipeline.step_indices.
+
+        With ``match_weights`` the batch also carries its samples' subisomorphisms (with the dummy column when
+        ``add_dummy``), and the match-weight targets are computed on the augmented batch in the same place: node weights
+        add no device->host read, edge weights the one of ``matching.edge_weights``."""
         counts = []
 
         def assemble():
-            p_dev, g_dev, c = ds.batch(idx)
+            if self.match_weights is None:
+                p_dev, g_dev, c = ds.batch(idx)
+                counts.append(c)
+                return self.transform(p_dev, g_dev)
+            from .subgraph_isomorphism import matching as M
+            p_dev, g_dev, c, sub = ds.batch(idx, subisomorphisms=True, dummy_column=self.add_dummy)
             counts.append(c)
-            return self.transform(p_dev, g_dev)
+            p_aug, g_aug = self.augment(p_dev, g_dev)
+            node, edge = self.match_weights
+            nw = M.node_weights_i32(sub, g_aug) if node else None
+            ew = M.edge_weights_i32(sub, p_aug, g_aug) if edge else None
+            return self._compile(p_aug, g_aug) + (nw, ew)
 
-        def train(graphs):
+        def train(out):
             if self.overlap:        # allocated on the transform stream, read by the train stream
                 counts[0].record_stream(torch.cuda.current_stream())
-            return self.train_on(*graphs, counts[0])
+            return self.train_on(out[0], out[1], counts[0], *out[2:])
 
         with self._global_batch(global_batch):
             if not self.overlap:

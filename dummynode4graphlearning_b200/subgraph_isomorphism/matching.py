@@ -42,15 +42,40 @@ def add_dummy_to_subisomorphisms(mats, graph_b):
     return out
 
 
+def dummy_column_offsets(val_sizes, rows):
+    """host int64 (B + 1) offsets of a packed subisomorphism batch after ``add_dummy_to_subisomorphisms``: sample b's
+    ``val_sizes[b]`` ids in ``rows[b]`` rows become ``val_sizes[b] + rows[b]`` ids."""
+    sizes = np.asarray(val_sizes, np.int64) + np.asarray(rows, np.int64)
+    out = np.zeros(len(sizes) + 1, dtype=np.int64)
+    np.cumsum(sizes, out=out[1:])
+    return out
+
+
+def append_dummy_column(subiso, graph_b, out_ptr, out_total):
+    """``add_dummy_to_subisomorphisms`` of a packed device batch (one launch, no device->host read): every row also maps
+    the pattern's dummy node to the graph's, whose graph-local id is the graph's node count in `graph_b`, the batch
+    BEFORE augmentation.  out_ptr: int32 device (B + 1) offsets of the result and out_total its last entry, both from
+    ``dummy_column_offsets`` on the host.  -> dict(val_ptr=out_ptr, values, rows) in the ``pack_subisomorphisms`` layout."""
+    from .. import ops
+    values = ops.subiso_append_dummy(subiso["val_ptr"], subiso["values"], subiso["rows"], graph_b["node_ptr"], out_ptr,
+                                     out_total)
+    return dict(val_ptr=out_ptr, values=values, rows=subiso["rows"])
+
+
 def node_weights(subiso, graph_b):
     """(N_g,) int64: number of subisomorphism entries that hit each graph node (zeros for samples without matches)."""
+    return node_weights_i32(subiso, graph_b).long()
+
+
+def node_weights_i32(subiso, graph_b):
+    """``node_weights`` as the kernel writes it (int32), what the fused match loss reads."""
     require_cuda(graph_b["src"], "graph batch")
     dev = graph_b["src"].device
     B, Ng = int(graph_b["num_graphs"]), int(graph_b["vlabel"].numel())
     w = torch.empty(Ng, dtype=torch.int32, device=dev)
     lib().call("dn4gl_subiso_node_weights", B, ptr(subiso["val_ptr"]), ptr(subiso["values"]), int(subiso["values"].numel()),
                ptr(graph_b["node_ptr"]), Ng, ptr(w), _stream())
-    return w.long()
+    return w
 
 
 def _sorted_out_lists(graph_b):
@@ -100,6 +125,11 @@ def conjugate_subisomorphisms(subiso, pattern_b, graph_b):
 def edge_weights(subiso, pattern_b, graph_b):
     """(E_g,) int64 in edge-id order: for every subisomorphism and pattern edge (u, v, l), +1 on every graph edge
     (map[u], map[v]) with label l -- with the reference's run/dict semantics for repeated pattern pairs."""
+    return edge_weights_i32(subiso, pattern_b, graph_b).long()
+
+
+def edge_weights_i32(subiso, pattern_b, graph_b):
+    """``edge_weights`` as the kernel writes it (int32); one device->host read (the work total)."""
     require_cuda(graph_b["src"], "graph batch")
     L = lib()
     dev = graph_b["src"].device
@@ -123,4 +153,4 @@ def edge_weights(subiso, pattern_b, graph_b):
            ptr(pattern_b["node_ptr"]), ptr(pattern_b["edge_ptr"]), ptr(pattern_b["src"]), ptr(pattern_b["dst"]),
            ptr(pattern_b["elabel"]), Ep, ptr(active), ptr(graph_b["node_ptr"]), ptr(csr.row_ptr), ptr(csr.eid),
            ptr(graph_b["dst"]), ptr(graph_b["elabel"]), Eg, ptr(w), _stream())
-    return w.long()
+    return w

@@ -244,6 +244,38 @@ int dn4gl_subiso_conjugate(int32_t B, const int32_t *work_ptr, int64_t total_wor
                            const int32_t *g_out_ptr, const int32_t *g_out_items, const int32_t *g_dst,
                            const int32_t *g_elabel, int32_t *conj, void *stream);
 
+/* The dummy column of add_dummy_nodes_edges (train.py:467-472), batched: row s of sample b (rows[b] rows of
+ * np_b = (val_ptr[b+1] - val_ptr[b]) / rows[b] ids) is written at out[out_ptr[b] + s * (np_b + 1)] as its np_b ids
+ * followed by n_b = g_node_ptr[b+1] - g_node_ptr[b], the graph's node count BEFORE augmentation (the graph-local id of
+ * the dummy node dn4gl_sub_add_dummy appends last).  Samples with rows[b] = 0 write nothing.  out_ptr[B+1]: the output
+ * offsets val_ptr[b] + sum_{b' < b} rows[b'] (from the caller's host size tables); out_total = out_ptr[B].          */
+int dn4gl_subiso_append_dummy(int32_t B, const int32_t *val_ptr, const int32_t *values, const int32_t *rows,
+                              const int32_t *g_node_ptr, const int32_t *out_ptr, int64_t out_total, int32_t *out,
+                              void *stream);
+
+/* The match terms of the counting models' bp_loss (train.py:776-813), node and edge kind in one launch each way
+ * (csrc/match.cu).  Per kind: pred[B*L] fp32 left-padded, mask[B*L] (bool bytes, 1 = real), w[N] int32 flat weights of
+ * the augmented graph batch with row offsets seg_ptr[B+1] (position (b, j) reads w[seg_ptr[b] + j - (L - len_b)] when
+ * j >= L - len_b); pred = NULL leaves the kind out.  On masked and padded positions prediction and target count as 0.
+ *   out[0] = (match_loss_w * sum crit(leaky(p, neg_slp) - w) + match_reg_w * sum crit(relu(p - pred_c[b]))) / B
+ * over both kinds' B*L positions; crit 0 = MAE, 1 = MSE, 2 = SMSE (smooth L1, beta 1).  neg_slp / match_loss_w /
+ * match_reg_w: device fp32 scalars.  Sums in double in an order fixed by B and the padded lengths; ws:
+ * dn4gl_match_loss_workspace_bytes(B) bytes, 8-byte aligned; counter: one int32 that is 0 on entry (left 0).
+ * The backward writes g_pred_v / g_pred_e (every position, masked and padded ones included) and g_pred_c[B] (the
+ * per-graph sum of the regulariser's derivatives) for the upstream gradient g_out[0].                              */
+size_t dn4gl_match_loss_workspace_bytes(int32_t B);
+int dn4gl_match_loss_f32(int32_t B, const float *pred_c, const float *pred_v, const uint8_t *mask_v, const int32_t *w_v,
+                         const int32_t *ptr_v, int32_t Lv, const float *pred_e, const uint8_t *mask_e,
+                         const int32_t *w_e, const int32_t *ptr_e, int32_t Le, int32_t crit, const float *neg_slp,
+                         const float *match_loss_w, const float *match_reg_w, float *out, void *ws, size_t ws_bytes,
+                         int32_t *counter, void *stream);
+int dn4gl_match_loss_bwd_f32(int32_t B, const float *g_out, const float *pred_c, const float *pred_v,
+                             const uint8_t *mask_v, const int32_t *w_v, const int32_t *ptr_v, int32_t Lv,
+                             const float *pred_e, const uint8_t *mask_e, const int32_t *w_e, const int32_t *ptr_e,
+                             int32_t Le, int32_t crit, const float *neg_slp, const float *match_loss_w,
+                             const float *match_reg_w, float *g_pred_v, float *g_pred_e, float *g_pred_c,
+                             void *stream);
+
 /* ---- a3: PyG read_tu_data canonicalisation ------------------------------------------------- */
 /* remove_self_loops + coalesce [torch-geometric 2.0.2 read_tu_data, called from
  * graph_classification/graph_neural_networks/dataset.py:151]: given the edge list's endpoints
